@@ -2,7 +2,7 @@
 """bench.py — routing decisions/s of the prefix-cache-aware Endpoint Picker hot path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--cfg 2|3|4|5] [--mode replicas|sharded] [--scale F]
+                    [--cfg 2|3|4|5] [--mode replicas|sharded] [--scale F] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path (hash → index lookup → weighted score → argmax)
 over one batch of synthetic requests.  Default workload = BASELINE.json's headline
@@ -38,6 +38,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from
 
 import numpy as np  # noqa: E402
 
@@ -558,6 +559,17 @@ class Scenario:
         avg = {k: (v[0] / v[1] if v[1] else 0.0) for k, v in kern.items()}
         return avg, st.probed_blocks / max(n, 1)
 
+    def last_picks(self, steps, pipelined):
+        """the picks [R, P] the last of `steps` timed steps wrote (run_steps: step i of the pipelined path writes
+        d_outs[i & 1], every stream-ordered step writes d_out)"""
+        import torch
+
+        from fusioninfer_b200 import PICK_DTYPE
+
+        buf = self.d_outs[(steps - 1) & 1] if pipelined else self.d_out
+        torch.cuda.synchronize()
+        return buf.cpu().numpy().view(PICK_DTYPE).reshape(self.wl.R, self.P)
+
     def picks_of_batch0(self):
         """the device path's picks of batch 0, as records [R, P] (+ the chains)"""
         import torch
@@ -633,6 +645,24 @@ def sub_record(sc, steps, warmup, peak, with_parity=True):
     return rec
 
 
+DUMP_BYTES = 60_000_000  # array data of --dump-outputs; with the .npy headers under 64 MB in all
+
+
+def dump_outputs(out_dir, picks):
+    """Write the picks [R, P] as DIR/<field>.npy (float64, exact for every field of fi_pick) plus DIR/request.npy,
+    the request index of each row.  Above DUMP_BYTES in all, the rows are a fixed seeded sample of the requests."""
+    R = picks.shape[0]
+    per_request = 8 * (1 + len(picks.dtype.names) * picks.shape[1])
+    rows = np.arange(R)
+    if R * per_request > DUMP_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(R, DUMP_BYTES // per_request, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "request.npy"), rows.astype(np.float64))
+    for name in picks.dtype.names:
+        np.save(os.path.join(out_dir, f"{name}.npy"), picks[rows][name].astype(np.float64))
+    log(f"picks of the last timed step ({len(rows)} of {R} requests) written to {out_dir}")
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -661,7 +691,13 @@ def main():
                     help="how the main run's index was built (the default run reports all three in roofline.index_order)")
     ap.add_argument("--churn-rounds", type=int, default=6, help="pick + indexer.Add rounds that age the 'churned' index")
     ap.add_argument("--extra-steps", type=int, default=30)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the picks of the last one as DIR/<field>.npy (float64; rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the picks of the GPU path (--impl ours)")
 
     from fusioninfer_b200 import synth
 
@@ -718,6 +754,8 @@ def main():
     ms_step, launches = sc.time_steps(args.steps, args.warmup, pipelined,
                                       clocks if (rank == 0 and os.environ.get("FI_BENCH_NO_CLOCKS") != "1") else None)
     clk = clocks.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, sc.last_picks(args.steps, pipelined))
     units = R * (world if mode == "replicas" else 1)
     value = units / (ms_step * 1e-3)
     stream_ordered = None

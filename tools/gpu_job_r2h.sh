@@ -1,6 +1,7 @@
 #!/bin/bash
 # r2h: hash_blocks on half-word arithmetic + 256-bit loads; chain-link variants microbenchmark; ncu full capture
 mkdir -p gpurun_out
+${NVCC:-/usr/local/cuda/bin/nvcc} -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -I fusioninfer_b200/csrc -o tools/microbench/chainlat tools/microbench/chainlat.cu || exit 1
 tools/microbench/chainlat > gpurun_out/r2h_chainlat.txt 2>&1; grep -a "hand\|manual\|pure_chain     grid  128 x  128" gpurun_out/r2h_chainlat.txt
 timeout 1200 python -m pytest tests/test_gpu_parity.py tests/test_gpu_fullsize.py -m gpu -q -x 2>&1 | tail -8 > gpurun_out/r2h_pytest.log; tail -3 gpurun_out/r2h_pytest.log
 for pl in "" "--no-pipeline"; do
