@@ -8,7 +8,8 @@ OBJDIR := build
 LIB := fusioninfer_b200/lib/libfi_epp.so
 HOSTCHECK := fusioninfer_b200/lib/libfi_hostcheck.so
 
-CU_SRCS := $(CSRC)/hash_kernels.cu $(CSRC)/index_kernels.cu $(CSRC)/lru_kernels.cu $(CSRC)/match_kernels.cu $(CSRC)/engine.cu
+CU_SRCS := $(CSRC)/hash_kernels.cu $(CSRC)/index_kernels.cu $(CSRC)/lru_kernels.cu $(CSRC)/match_kernels.cu \
+           $(CSRC)/engine.cu $(CSRC)/engine_index.cu $(CSRC)/engine_lru.cu $(CSRC)/engine_pick.cu $(CSRC)/engine_comm.cu
 CU_OBJS := $(patsubst $(CSRC)/%.cu,$(OBJDIR)/%.o,$(CU_SRCS))
 HDRS := $(wildcard $(CSRC)/*.cuh) $(wildcard $(CSRC)/*.h) include/fi_epp.h
 
@@ -45,7 +46,7 @@ TIMING_LIB := fusioninfer_b200/lib/libfi_epp_timing.so
 timing: $(TIMING_LIB)
 $(TIMING_LIB): $(CU_SRCS) $(HDRS) $(OBJDIR)/epp_config.o
 	@mkdir -p $(OBJDIR)/timing
-	for f in hash_kernels index_kernels lru_kernels match_kernels engine; do $(NVCC) $(ARCH) -O3 -std=c++17 -lineinfo -DFI_MATCH_TIMING -Xcompiler -fPIC -c $(CSRC)/$$f.cu -o $(OBJDIR)/timing/$$f.o || exit 1; done
+	for f in hash_kernels index_kernels lru_kernels match_kernels engine engine_index engine_lru engine_pick engine_comm; do $(NVCC) $(ARCH) -O3 -std=c++17 -lineinfo -DFI_MATCH_TIMING -Xcompiler -fPIC -c $(CSRC)/$$f.cu -o $(OBJDIR)/timing/$$f.o || exit 1; done
 	$(NVCC) $(ARCH) -shared -o $@ $(OBJDIR)/timing/*.o $(OBJDIR)/epp_config.o -ldl
 .PHONY: timing
 
@@ -53,6 +54,6 @@ $(TIMING_LIB): $(CU_SRCS) $(HDRS) $(OBJDIR)/epp_config.o
 # -> fusioninfer_b200/lib/libfi_epp_$(NAME).so (select it with FI_EPP_LIB=<path>)
 variant: $(CU_SRCS) $(HDRS) $(OBJDIR)/epp_config.o
 	@mkdir -p $(OBJDIR)/$(NAME)
-	for f in hash_kernels index_kernels lru_kernels match_kernels engine; do $(NVCC) $(ARCH) -O3 -std=c++17 -lineinfo $(DEFS) -Xcompiler -fPIC -c $(CSRC)/$$f.cu -o $(OBJDIR)/$(NAME)/$$f.o || exit 1; done
+	for f in hash_kernels index_kernels lru_kernels match_kernels engine engine_index engine_lru engine_pick engine_comm; do $(NVCC) $(ARCH) -O3 -std=c++17 -lineinfo $(DEFS) -Xcompiler -fPIC -c $(CSRC)/$$f.cu -o $(OBJDIR)/$(NAME)/$$f.o || exit 1; done
 	$(NVCC) $(ARCH) -shared -o fusioninfer_b200/lib/libfi_epp_$(NAME).so $(OBJDIR)/$(NAME)/*.o $(OBJDIR)/epp_config.o -ldl
 .PHONY: variant

@@ -1,366 +1,12 @@
-// engine.cu — host side of libfi_epp: the C ABI of include/fi_epp.h.
-//
-// Owns the device buffers, two CUDA streams (compute, index maintenance),
-// the pinned op ring that keeps the GPU index live (async H2D on the side stream,
-// ordered before the next pick), the host LRU, the per-batch score tables, and the
-// optional NCCL communicator for endpoint-range sharded pools.  No CPU fallback:
-// creation fails without a CUDA device.
-#include <cuda.h>  // types and prototypes of the green-context API only: reached through cudaGetDriverEntryPoint, libcuda is not linked
-#include <cuda_runtime.h>
-#include <unistd.h>
-#include <dlfcn.h>
+// engine.cu — host side of libfi_epp (handle and parts: engine.h): create, destroy, options, stats, other entry points.
+#include "engine.h"
 
-#include <algorithm>
-#include <atomic>
-#include <chrono>
-#include <cmath>
-#include <condition_variable>
-#include <cstdio>
-#include <cstdlib>
-#include <cstring>
-#include <functional>
-#include <memory>
-#include <mutex>
-#include <string>
-#include <thread>
-#include <unordered_set>
-#include <vector>
-
-#include <sched.h>
-
-#include "../../include/fi_epp.h"
-#include "kernels.cuh"
-#include "lru.h"
-#include "lru_batch.h"
-#include "lru_device.cuh"
-#include "lru_plan.h"
-#include "xxh64.cuh"
-
-using namespace fi;
-
-namespace {
-
-// ---- minimal NCCL binding through dlopen (the torch-bundled or the system libnccl.so.2) ----
-typedef struct ncclComm* ncclComm_t;
-typedef struct {
-  char internal[128];
-} ncclUniqueId;
-enum { ncclSuccess = 0 };
-enum { ncclInt8 = 0, ncclChar = 0, ncclUint8 = 1 };
-struct NcclApi {
-  void* lib = nullptr;
-  int (*GetUniqueId)(ncclUniqueId*) = nullptr;
-  int (*CommInitRank)(ncclComm_t*, int, ncclUniqueId, int) = nullptr;
-  int (*CommDestroy)(ncclComm_t) = nullptr;
-  int (*AllGather)(const void*, void*, size_t, int, ncclComm_t, cudaStream_t) = nullptr;
-  const char* (*GetErrorString)(int) = nullptr;
-  bool load(std::string* err) {
-    if (lib) return true;
-    const char* names[] = {"libnccl.so.2", "libnccl.so"};
-    for (const char* n : names) {
-      lib = dlopen(n, RTLD_NOW | RTLD_GLOBAL);
-      if (lib) break;
-    }
-    if (!lib) {
-      *err = std::string("dlopen libnccl.so.2 failed: ") + dlerror();
-      return false;
-    }
-    GetUniqueId = (decltype(GetUniqueId))dlsym(lib, "ncclGetUniqueId");
-    CommInitRank = (decltype(CommInitRank))dlsym(lib, "ncclCommInitRank");
-    CommDestroy = (decltype(CommDestroy))dlsym(lib, "ncclCommDestroy");
-    AllGather = (decltype(AllGather))dlsym(lib, "ncclAllGather");
-    GetErrorString = (decltype(GetErrorString))dlsym(lib, "ncclGetErrorString");
-    if (!GetUniqueId || !CommInitRank || !CommDestroy || !AllGather) {
-      *err = "libnccl is missing a required symbol";
-      return false;
-    }
-    return true;
-  }
-};
-NcclApi g_nccl;
-std::mutex g_nccl_mu;
-
-struct PairKey {
-  uint64_t hash;
-  uint32_t endpoint;
-  bool operator==(const PairKey& o) const { return hash == o.hash && endpoint == o.endpoint; }
-};
-struct PairHash {
-  size_t operator()(const PairKey& k) const {
-    uint64_t x = k.hash ^ ((uint64_t)k.endpoint * 0x9E3779B97F4A7C15ULL);
-    x ^= x >> 29;
-    return (size_t)(x * 0xBF58476D1CE4E5B9ULL);
-  }
-};
-
-constexpr uint64_t kOpChunk = 1ull << 20;  // ops per pinned staging buffer
-
-enum KernelKind { K_HASH = 0, K_CHAIN = 1, K_MATCH = 2, K_INDEX = 3, K_OTHER = 4, K_KINDS = 5 };
-
-uint32_t pow2_ceil32(uint32_t v) {
-  uint32_t p = 1;
-  while (p < v) p <<= 1;
-  return p;
-}
-uint64_t pow2_ceil64(uint64_t v) {
-  uint64_t p = 1;
-  while (p < v) p <<= 1;
-  return p;
-}
-
-// host cores this process may really use: the affinity mask capped by the cgroup CPU quota (more runnable
-// threads than quota only get the group throttled)
-unsigned usable_cores() {
-  unsigned n = std::thread::hardware_concurrency();
-  cpu_set_t set;
-  CPU_ZERO(&set);
-  if (sched_getaffinity(0, sizeof(set), &set) == 0 && CPU_COUNT(&set) > 0) n = (unsigned)CPU_COUNT(&set);
-  if (FILE* f = std::fopen("/sys/fs/cgroup/cpu.max", "r")) {  // cgroup v2: "<quota|max> <period>"
-    char q[64] = {0};
-    long long period = 0;
-    if (std::fscanf(f, "%63s %lld", q, &period) == 2 && std::strcmp(q, "max") != 0 && period > 0) {
-      const long long quota = std::atoll(q);
-      if (quota > 0) n = std::min<unsigned>(n, (unsigned)std::max<long long>(1, (quota + period - 1) / period));
-    }
-    std::fclose(f);
-  }
-  return n ? n : 1u;
-}
-
-}  // namespace
-
-struct fi_epp {
-  fi_epp_config cfg;
-  std::mutex mu;
-  std::string err;
-  int sm_count = 148;
-  uint32_t MP = 0;  // chain pitch
-  uint32_t W = 0;   // words per index row
-  uint32_t P = 0;   // profiles
-  bool fast_hash = false;
-
-  cudaStream_t s_main = nullptr, s_index = nullptr;  // compute; index maintenance (side stream)
-  // host-buffer picks feed the prompts in slices: the copy engine runs ahead on s_copy while s_main hashes,
-  // walks and matches the slices that have landed (the step is PCIe-bound: only the last slice's work is exposed)
-  cudaStream_t s_copy = nullptr;
-  static constexpr int kMaxFeedSlices = 16;
-  cudaEvent_t ev_copy[kMaxFeedSlices] = {};
-  uint32_t feed_slices = 8;  // FI_EPP_FEED_SLICES (1: one copy, then the whole batch)
-  // Pipelined device path (fi_epp_pick_submit / fi_epp_pick_wait): stage A (block hashing + chain walk) of
-  // batch k+1 runs on s_a while stage B (match + pick) of batch k runs on s_main; the chain / block-count
-  // buffers are double-buffered (slot = batch parity), the pre-states are not (stage A is serial on s_a).
-  cudaStream_t s_a = nullptr;
-  uint64_t* d_chain2 = nullptr;
-  uint32_t* d_nblocks2 = nullptr;
-  cudaEvent_t ev_in = nullptr, ev_a[2] = {}, ev_b[2] = {};
-  cudaEvent_t ev_pick = nullptr;   // completion of the most recent pick of any kind: ev_pick_own, or (partitioned
-                                   // pipeline) the slot event of the batch submitted last — a handle, not a second record
-  cudaEvent_t ev_pick_own = nullptr;
-  cudaEvent_t ev_plain = nullptr;  // completion of the most recent stream-ordered (not pipelined) pick
-  uint64_t pipe_seq = 0;          // batches submitted
-  uint32_t pipe_hash_ctas = 0;    // per-SM caps of the pipelined path's two co-running kernels (0 = uncapped);
-  uint32_t pipe_match_ctas = 0;   // FI_EPP_PIPE_HASH_CTAS / FI_EPP_PIPE_MATCH_CTAS, option "pipe_hash_ctas" / "pipe_match_ctas"
-  // SM-partitioned pipeline (green contexts, CUDA 12.4+): the chain walk is serial latency that fills 6 % of the
-  // warp slots but cannot share schedulers with a busy kernel (it slows 3x), so nothing overlapped it and every
-  // batch paid its 27 us.  With the GPU split into a 40-SM partition for the walker (three or four of its warps per
-  // scheduler) and a 108-SM partition for hash_blocks / match_pick, batch k is matched while batch k+1's chains
-  // are walked and batch k+2 is hashed: three batches in flight, 131 -> 116 us per batch.
-  // FI_EPP_PIPE_PARTITION=<SMs> / option "pipe_partition" (0 = off: two batches in flight on the whole GPU).
-  // SMs asked for the walker partition.  Measured at cfg 3 (us per step; no partition: 131.1): 8 -> 240, 16 -> 125.6,
-  // 24 -> 123.0, 32 -> 129.0, 40 -> 116.2 (three runs), 48 -> 124.3, 56 -> 133.7
-  int part_want = 40;
-  int part_compact = -1;        // walker shape on the partition: -1 = the 64-register shape only where the 78-register one does
-                                // not fit (fewer than 24 SMs); FI_EPP_WALK_COMPACT=0/1 forces it
-  int part_state = 0;           // 0: not tried, 1: active, -1: unavailable (fallback to the unpartitioned pipeline)
-  bool part_active = false;     // the partitioned pipeline has batches in flight / owns the slot events
-  // how often ev_index / ev_plain / ev_lru have been re-recorded, and the values the partitioned pipeline's streams
-  // already waited for: a submit makes ~16 runtime calls instead of ~23 (eight processes on a 16-core host are
-  // launch-bound otherwise)
-  uint64_t gen_index = 0, gen_plain = 0, gen_lru = 0;
-  uint64_t seen_index = ~0ull, seen_plain = ~0ull, seen_lru = ~0ull;
-  uint64_t part_seq = 0;        // batches submitted to it since it last became active
-  int part_walk_sms = 0, part_main_sms = 0;
-  CUgreenCtx gctx_walk = nullptr, gctx_main = nullptr;
-  cudaStream_t s_pw = nullptr, s_pa = nullptr, s_pb = nullptr;  // walker | hashing, matching (big partition)
-  uint64_t* d_pre2 = nullptr;
-  uint32_t* d_nblocks3 = nullptr;
-  cudaEvent_t ev_h[2] = {}, ev_b3[3] = {}, ev_up = nullptr;
-  cudaEvent_t ev_index = nullptr, ev_user = nullptr, ev_done = nullptr, ev_ctr = nullptr;
-
-  // request buffers (device)
-  uint8_t* d_prompts = nullptr;
-  uint64_t* d_offsets = nullptr;
-  uint64_t* d_h0 = nullptr;
-  uint64_t* d_pre = nullptr;
-  uint64_t* d_chain = nullptr;
-  uint32_t* d_nblocks = nullptr;
-  fi_pick* d_picks = nullptr;   // [R][P] final
-  fi_pick* d_local = nullptr;   // [R][P] this rank's picks (sharded)
-  fi_pick* d_gather = nullptr;  // [world][R][P]
-  // peer-memory exchange (sharded mode; kernels.cuh PeerXchg)
-  PeerXchg px{};                 // px.enabled == 0: NCCL all-gathers are used
-  uint8_t* d_xchg = nullptr;     // this rank's exchange buffer
-  volatile uint32_t* h_xerr = nullptr;  // poll-timeout flag of the exchange (mapped pinned host word the kernels set)
-  void* peer_ipc[FI_MAX_RANKS] = {};  // mappings opened with cudaIpcOpenMemHandle (closed in destroy)
-  // sharded mode: every rank hashes every prompt (the default: 149 vs 141 M decisions/s at cfg 4 on 8 GPUs, 131 vs
-  // 119 on 2 — hashing 16 KiB from local HBM costs less than receiving 2 KiB of chain over NVLink); FI_EPP_SHARD_HASH=
-  // split / option "shard_hash" = 1: every rank hashes R/world requests and the chains are all-gathered
-  bool split_hash = false;
-  uint32_t chain_rows = 0;  // rows allocated in d_chain / d_pre / d_nblocks (max_batch padded for the gather)
-  // sharded mode: directory gossip (index_kernels.cu): this rank's transition log of the current round and the
-  // buffers the ranks' logs are gathered into
-  unsigned long long* d_glog_n = nullptr;  // [2] appear / vanish counts
-  uint64_t* d_glog_a = nullptr;            // [kOpChunk]
-  uint64_t* d_glog_v = nullptr;            // [kOpChunk]
-  unsigned long long* d_ghdr = nullptr;    // [world][2] gathered counts
-  unsigned long long* h_ghdr = nullptr;    // pinned copy
-  uint64_t* d_ggather = nullptr;           // [world][kOpChunk]
-  unsigned long long* d_probed = nullptr;
-  uint32_t* d_work = nullptr;  // [16] dynamic work-queue counters of in-flight match launches
-  // pinned host mirrors
-  fi_pick* h_picks = nullptr;
-  uint64_t* h_offsets = nullptr;
-  uint64_t* h_h0 = nullptr;
-  uint32_t* h_nblocks = nullptr;
-
-  // index
-  IndexView ix{};
-  IndexView ix_spare{};  // rebuild target, allocated at the first rebuild and reused alternately
-  bool spare_ready = false;
-  IndexCounters* d_ctr = nullptr;
-  IndexCounters* h_ctr = nullptr;  // pinned
-  bool ctr_pending = false;
-  uint64_t rebuilds = 0, ops_applied = 0;
-  fi_index_op* h_sets[2] = {nullptr, nullptr};
-  fi_index_op* h_clears[2] = {nullptr, nullptr};
-  fi_index_op* d_sets[2] = {nullptr, nullptr};
-  fi_index_op* d_clears[2] = {nullptr, nullptr};
-  cudaEvent_t ev_buf[2] = {nullptr, nullptr};
-  int cur_buf = 0;
-  uint64_t n_sets = 0, n_clears = 0;
-  std::unordered_set<PairKey, PairHash> cleared;
-  LruArena lru_arena;  // backing store of the LRUs (one huge-page mapping)
-  std::vector<LruSet> lrus;
-  std::unique_ptr<WorkerPool> pool;  // host LRU workers (fi_epp_index_add_chains), created on first use
-  std::vector<WorkerOps> lru_outs;   // their op lists (capacity kept from batch to batch)
-  bool verbose = false;              // FI_EPP_VERBOSE
-  // device-resident LRU (lru_kernels.cu): the default for single-rank handles whose lru_capacity holds a whole
-  // chain; option "device_lru" / FI_EPP_DEVICE_LRU=0 selects the host LRU instead.  Allocated at the first Add;
-  // the two are never mixed on one handle.
-  int lru_mode = -1;  // -1: not chosen yet, 0: host LRU, 1: device LRU
-  int lru_want = -1;  // option / environment override (-1: automatic)
-  bool dlru_ready = false;  // the device LRU's buffers are all there
-  uint32_t lru_table_slots = 0;  // option "lru_table_slots": slots per endpoint table of the device LRU (0: sized by free HBM)
-  DevLru dlru{};
-  uint32_t* d_lru_state = nullptr;           // head | tail | count | used | error
-  unsigned long long* d_lru_ctr = nullptr;   // [0] SETs emitted, [1] endpoints maintained, [2] CLEARs of the running sub-batch,
-                                             // [3] CLEARs total, [4] doomed winners
-  struct LruHostStat {
-    uint32_t error, any_ovf;  // (any_ovf: the touch kernel's overflow flag of the running sub-batch)
-    unsigned long long n_sets, n_maintained, n_clears_cur, n_clears, n_doomed;
-  };
-  uint64_t lru_deferred = 0, lru_sub_batches = 0;  // host-side totals
-  LruHostStat* h_lru_stat = nullptr;         // pinned copy, refreshed after every call
-  uint32_t* d_lru_plan = nullptr;            // the planner's arrays of the current call
-  uint32_t* h_lru_plan = nullptr;            // pinned staging of the same
-  size_t lru_plan_cap = 0;                   // in u32 words
-  uint32_t *d_lru_slot_of = nullptr, *d_lru_wcount = nullptr, *d_lru_base = nullptr;
-  fi_index_op *d_lru_sets = nullptr, *d_lru_clears = nullptr;
-  uint64_t lru_touch_cap = 0;                // touches per sub-batch the scratch arrays hold
-  uint64_t* d_lru_chains = nullptr;          // staging of host chains
-  size_t lru_chains_cap = 0;                 // in u64 words
-  cudaEvent_t ev_lru = nullptr;              // the previous call's staging has been consumed
-  cudaEvent_t ev_lru_ovf = nullptr;          // the touch kernel's overflow flag has reached the host
-  uint32_t last_plain_R = 0;                 // rows of d_chain the most recent stream-ordered pick wrote
-  LruPlan lru_plan;
-  unsigned lru_threads = 0;          // 0: FI_EPP_LRU_THREADS, else min(usable cores, 64)
-
-  // endpoints / score tables
-  std::vector<EndpointDev> eps;  // global pool
-  bool eps_dirty = true;
-  EndpointDev* d_eps = nullptr;
-  double* d_sc = nullptr;
-  uint32_t* d_elig = nullptr;
-  ZeroBest* d_zero = nullptr;
-  uint32_t* d_ztie = nullptr;
-  std::vector<LoraDev> lora;   // local endpoints' adapter residency (lora-affinity-scorer)
-  bool lora_dirty = false;
-  LoraDev* d_lora = nullptr;
-  uint64_t* d_adapters = nullptr;  // staging of the host path's per-request adapter ids
-  uint64_t* h_adapters = nullptr;  // pinned
-  ScoreTables st{};
-
-  // multi-GPU
-  ncclComm_t comm = nullptr;
-  uint32_t rank = 0, world = 1;
-
-  // stats / profiling
-  fi_epp_stats stats{};
-  bool profiling = false;
-  bool tracing = false;       // FI_EPP_TRACE=<call index>: print that call's kernel timeline to stderr
-  long trace_call = -1;
-  cudaEvent_t ev_trace0 = nullptr;
-  struct Ev {
-    cudaEvent_t a, b;
-    int kind;
-  };
-  std::vector<Ev> pending_ev;
-  std::vector<cudaEvent_t> ev_pool;
-};
-
-namespace {
-
-#define FI_CUDA(call)                                                                   \
-  do {                                                                                  \
-    cudaError_t e__ = (call);                                                           \
-    if (e__ != cudaSuccess) {                                                           \
-      h->err = std::string(#call) + ": " + cudaGetErrorString(e__);                     \
-      return FI_ERR_CUDA;                                                               \
-    }                                                                                   \
-  } while (0)
-
-int fail(fi_epp* h, int code, const std::string& m) {
-  h->err = m;
-  return code;
-}
-
-cudaEvent_t get_event(fi_epp* h) {
-  if (!h->ev_pool.empty()) {
-    cudaEvent_t e = h->ev_pool.back();
-    h->ev_pool.pop_back();
-    return e;
-  }
-  cudaEvent_t e = nullptr;
-  cudaEventCreate(&e);
-  return e;
-}
-
-// wraps one kernel launch: counts it and, when profiling, brackets it with events
-struct LaunchScope {
-  fi_epp* h;
-  cudaStream_t s;
-  int kind;
-  cudaEvent_t a = nullptr, b = nullptr;
-  LaunchScope(fi_epp* h_, cudaStream_t s_, int kind_) : h(h_), s(s_), kind(kind_) {
-    h->stats.kernel_launches++;
-    if (h->profiling || h->tracing) {
-      a = get_event(h);
-      b = get_event(h);
-      cudaEventRecord(a, s);
-    }
-  }
-  ~LaunchScope() {
-    if (h->profiling || h->tracing) {
-      cudaEventRecord(b, s);
-      h->pending_ev.push_back({a, b, kind});
-    }
-  }
-};
+namespace fi {
 
 void drain_profile(fi_epp* h) {
   for (auto& e : h->pending_ev) {
     float ms = 0.f;
-    if (cudaEventSynchronize(e.b) == cudaSuccess && cudaEventElapsedTime(&ms, e.a, e.b) == cudaSuccess) {
+    if (cudaEventSynchronize(e.b.get()) == cudaSuccess && cudaEventElapsedTime(&ms, e.a.get(), e.b.get()) == cudaSuccess) {
       switch (e.kind) {
         case K_HASH: h->stats.ms_hash_blocks += ms; h->stats.n_hash_blocks++; break;
         case K_CHAIN: h->stats.ms_chain_probe += ms; h->stats.n_chain_probe++; break;
@@ -369,1231 +15,10 @@ void drain_profile(fi_epp* h) {
         default: h->stats.ms_other += ms; h->stats.n_other++; break;
       }
     }
-    h->ev_pool.push_back(e.a);
-    h->ev_pool.push_back(e.b);
+    h->ev_pool.push_back(std::move(e.a));
+    h->ev_pool.push_back(std::move(e.b));
   }
   h->pending_ev.clear();
-}
-
-void free_index(IndexView& v) {
-  cudaFree(v.keys);
-  cudaFree(v.node_of);
-  cudaFree(v.klog);
-  cudaFree(v.rows);
-  cudaFree(v.cnt);
-  cudaFree(v.rmask);
-  v.keys = nullptr;
-  v.node_of = nullptr;
-  v.klog = nullptr;
-  v.rows = nullptr;
-  v.cnt = nullptr;
-  v.rmask = nullptr;
-}
-
-size_t index_bytes(uint64_t slots, uint32_t W) {
-  const uint64_t total = slots + 3;
-  return total * (sizeof(uint64_t) * 2 + sizeof(uint32_t) * 3 + (size_t)W * sizeof(uint32_t));
-}
-
-// queue the clears that make `v` an empty index (on the index stream)
-int clear_index(fi_epp* h, IndexView& v) {
-  const uint64_t total = v.C + 3;
-  FI_CUDA(cudaMemsetAsync(v.keys, 0, total * sizeof(uint64_t), h->s_index));
-  FI_CUDA(cudaMemsetAsync(v.node_of, 0xFF, total * sizeof(uint32_t), h->s_index));  // NODE_INVALID
-  FI_CUDA(cudaMemsetAsync(v.klog, 0, total * sizeof(uint64_t), h->s_index));
-  FI_CUDA(cudaMemsetAsync(v.rows, 0, total * v.W * sizeof(uint32_t), h->s_index));
-  FI_CUDA(cudaMemsetAsync(v.cnt, 0, total * sizeof(uint32_t), h->s_index));
-  FI_CUDA(cudaMemsetAsync(v.rmask, 0, total * sizeof(uint32_t), h->s_index));
-  return FI_OK;
-}
-
-int alloc_index(fi_epp* h, uint64_t slots, IndexView* out) {
-  IndexView v{};
-  v.C = slots;
-  v.bmask = slots / BUCKET_KEYS - 1;
-  v.W = h->W;
-  v.logW = 0;
-  while ((1u << v.logW) < v.W) ++v.logW;
-  const uint64_t total = slots + 3;  // + slots for hash 0, hash ~0, and a permanently-zero row
-  size_t free_b = 0, total_b = 0;
-  if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess && index_bytes(slots, v.W) + (256ull << 20) > free_b) {
-    h->err = "index of " + std::to_string(index_bytes(slots, v.W) >> 20) + " MiB does not fit in the " +
-             std::to_string(free_b >> 20) + " MiB of free device memory";
-    return FI_ERR_NOMEM;
-  }
-  cudaError_t e = cudaMalloc(&v.keys, total * sizeof(uint64_t));
-  if (e == cudaSuccess) e = cudaMalloc(&v.node_of, total * sizeof(uint32_t));
-  if (e == cudaSuccess) e = cudaMalloc(&v.klog, total * sizeof(uint64_t));
-  if (e == cudaSuccess) e = cudaMalloc(&v.rows, total * v.W * sizeof(uint32_t));
-  if (e == cudaSuccess) e = cudaMalloc(&v.cnt, total * sizeof(uint32_t));
-  if (e == cudaSuccess) e = cudaMalloc(&v.rmask, total * sizeof(uint32_t));
-  if (e != cudaSuccess) {  // nothing of a partial view survives
-    cudaGetLastError();
-    free_index(v);
-    h->err = std::string("index allocation: ") + cudaGetErrorString(e);
-    return e == cudaErrorMemoryAllocation ? FI_ERR_NOMEM : FI_ERR_CUDA;
-  }
-  int rc = clear_index(h, v);
-  if (rc != FI_OK) {
-    free_index(v);
-    return rc;
-  }
-  *out = v;
-  return FI_OK;
-}
-
-// Compact the live nodes into the spare table and swap.  Everything is queued on the index stream — no host
-// synchronisation: picks submitted later wait for ev_index (recorded by the flush that called us) and are
-// launched with the new view; picks already in flight keep reading the old tables, which are not touched again
-// before the NEXT rebuild, and that one is ordered behind them (flush_ops makes s_index wait for ev_pick).
-// The spare is allocated once, at the first rebuild (the only point where memory doubles), and then reused.
-int rebuild_index(fi_epp* h) {
-  if (!h->spare_ready) {
-    int rc = alloc_index(h, h->ix.C, &h->ix_spare);  // clears it too
-    if (rc != FI_OK) return rc;
-    h->spare_ready = true;
-  } else {
-    int rc = clear_index(h, h->ix_spare);
-    if (rc != FI_OK) return rc;
-  }
-  FI_CUDA(cudaMemsetAsync(h->d_ctr, 0, sizeof(IndexCounters), h->s_index));
-  {
-    LaunchScope ls(h, h->s_index, K_INDEX);
-    FI_CUDA(launch_index_rebuild(h->ix, h->ix_spare, h->d_ctr, h->s_index));
-  }
-  std::swap(h->ix, h->ix_spare);
-  h->rebuilds++;
-  return FI_OK;
-}
-
-// look at the counters copied back after the previous flush; rebuild if the table is
-// clogged with tombstones, fail if it is genuinely full
-int check_counters(fi_epp* h) {
-  if (!h->ctr_pending) return FI_OK;
-  FI_CUDA(cudaEventSynchronize(h->ev_ctr));
-  h->ctr_pending = false;
-  if (h->h_lru_stat && h->h_lru_stat->error)
-    return fail(h, FI_ERR_STATE, "device LRU: invariant " + std::to_string(h->h_lru_stat->error) + " broken");
-  if (h->h_ctr->overflow) return fail(h, FI_ERR_CAPACITY, "index full: raise index_slots");
-  const uint64_t used = h->h_ctr->used, tomb = h->h_ctr->tombstones;
-  if (used * 10 > h->ix.C * 7) {
-    if ((used - tomb) * 10 > h->ix.C * 6) return fail(h, FI_ERR_CAPACITY, "index above 60% live keys: raise index_slots");
-    // the rebuild reads the old tables on s_index: every pick that still uses them must be ordered before the
-    // NEXT rebuild clears them — flush_ops (our only caller that launches work) waits for ev_pick first
-    FI_CUDA(cudaStreamWaitEvent(h->s_index, h->ev_pick, 0));
-    int rc = rebuild_index(h);
-    if (rc != FI_OK) return rc;
-    FI_CUDA(cudaEventRecord(h->ev_index, h->s_index));
-  h->gen_index++;
-  }
-  return FI_OK;
-}
-
-GossipLog gossip_log(fi_epp* h) {
-  GossipLog g{};
-  if (h->world > 1) {
-    g.n_appear = h->d_glog_n;
-    g.n_vanish = h->d_glog_n + 1;
-    g.appear = h->d_glog_a;
-    g.vanish = h->d_glog_v;
-    g.cap = kOpChunk;
-  }
-  return g;
-}
-
-// launch the staged SET then CLEAR ops of the current group on the index stream.
-// Asynchronous: the only waits are for the *previous* group's counters (rebuild /
-// overflow decisions lag one group) and for the staging buffer being reused.
-int flush_ops(fi_epp* h) {
-  if (h->n_sets == 0 && h->n_clears == 0) return FI_OK;
-  int rc = check_counters(h);  // may rebuild (swaps tables) — only ever between groups
-  if (rc != FI_OK) return rc;
-  const int b = h->cur_buf;
-  // ops submitted after a pick returned must not overtake it on the GPU: the pick sees the index as of its call
-  FI_CUDA(cudaStreamWaitEvent(h->s_index, h->ev_pick, 0));
-  const GossipLog gl = gossip_log(h);
-  if (h->n_sets) {
-    FI_CUDA(cudaMemcpyAsync(h->d_sets[b], h->h_sets[b], h->n_sets * sizeof(fi_index_op), cudaMemcpyHostToDevice, h->s_index));
-    h->stats.h2d_bytes += h->n_sets * sizeof(fi_index_op);
-    LaunchScope ls(h, h->s_index, K_INDEX);
-    FI_CUDA(launch_index_set(h->ix, h->d_ctr, h->d_sets[b], h->n_sets, h->cfg.endpoint_begin, h->cfg.endpoint_count, h->rank,
-                             gl, h->s_index));
-  }
-  if (h->n_clears) {
-    FI_CUDA(cudaMemcpyAsync(h->d_clears[b], h->h_clears[b], h->n_clears * sizeof(fi_index_op), cudaMemcpyHostToDevice, h->s_index));
-    h->stats.h2d_bytes += h->n_clears * sizeof(fi_index_op);
-    LaunchScope ls(h, h->s_index, K_INDEX);
-    FI_CUDA(launch_index_clear(h->ix, h->d_ctr, h->d_clears[b], h->n_clears, h->cfg.endpoint_begin, h->cfg.endpoint_count,
-                               h->rank, gl, h->s_index));
-  }
-  h->ops_applied += h->n_sets + h->n_clears;
-  FI_CUDA(cudaEventRecord(h->ev_buf[b], h->s_index));
-  FI_CUDA(cudaMemcpyAsync(h->h_ctr, h->d_ctr, sizeof(IndexCounters), cudaMemcpyDeviceToHost, h->s_index));
-  FI_CUDA(cudaEventRecord(h->ev_ctr, h->s_index));
-  h->ctr_pending = true;
-  FI_CUDA(cudaEventRecord(h->ev_index, h->s_index));
-  h->gen_index++;
-  h->n_sets = h->n_clears = 0;
-  h->cleared.clear();
-  h->cur_buf ^= 1;
-  // the buffer we are about to fill must have been consumed
-  FI_CUDA(cudaEventSynchronize(h->ev_buf[h->cur_buf]));
-  return FI_OK;
-}
-
-int nccl_allgather_on(fi_epp* h, const void* send, void* recv, size_t bytes, cudaStream_t s);
-
-// Sharded pools, one gossip round (collective: every rank calls it the same number of times): exchange the
-// transition logs written by this round's SET / CLEAR kernels and replay the other ranks' into the local
-// directory — all APPEARs before all VANISHes, like the SETs and CLEARs that produced them.
-int gossip_round(fi_epp* h) {
-  if (h->world <= 1) return FI_OK;
-  const uint32_t Wd = h->world;
-  int rc = nccl_allgather_on(h, h->d_glog_n, h->d_ghdr, 2 * sizeof(unsigned long long), h->s_index);
-  if (rc != FI_OK) return rc;
-  FI_CUDA(cudaMemcpyAsync(h->h_ghdr, h->d_ghdr, (size_t)Wd * 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->s_index));
-  FI_CUDA(cudaStreamSynchronize(h->s_index));
-  uint64_t na = 0, nv = 0;
-  for (uint32_t g = 0; g < Wd; ++g) {
-    na = std::max<uint64_t>(na, h->h_ghdr[2 * g]);
-    nv = std::max<uint64_t>(nv, h->h_ghdr[2 * g + 1]);
-  }
-  if (na > kOpChunk || nv > kOpChunk) return fail(h, FI_ERR_STATE, "gossip log overflow");
-  if (na) {
-    rc = nccl_allgather_on(h, h->d_glog_a, h->d_ggather, na * sizeof(uint64_t), h->s_index);
-    if (rc != FI_OK) return rc;
-    for (uint32_t g = 0; g < Wd; ++g) {
-      if (g == h->rank || h->h_ghdr[2 * g] == 0) continue;
-      LaunchScope ls(h, h->s_index, K_INDEX);
-      FI_CUDA(launch_index_remote_appear(h->ix, h->d_ctr, h->d_ggather + (size_t)g * na, h->h_ghdr[2 * g], g, h->s_index));
-    }
-  }
-  if (nv) {
-    rc = nccl_allgather_on(h, h->d_glog_v, h->d_ggather, nv * sizeof(uint64_t), h->s_index);
-    if (rc != FI_OK) return rc;
-    for (uint32_t g = 0; g < Wd; ++g) {
-      if (g == h->rank || h->h_ghdr[2 * g + 1] == 0) continue;
-      LaunchScope ls(h, h->s_index, K_INDEX);
-      FI_CUDA(launch_index_remote_vanish(h->ix, h->d_ctr, h->d_ggather + (size_t)g * nv, h->h_ghdr[2 * g + 1], g, h->s_index));
-    }
-  }
-  FI_CUDA(cudaMemsetAsync(h->d_glog_n, 0, 2 * sizeof(unsigned long long), h->s_index));
-  if (na || nv) {  // the replays allocate nodes too: refresh the counters the rebuild decision reads
-    FI_CUDA(cudaMemcpyAsync(h->h_ctr, h->d_ctr, sizeof(IndexCounters), cudaMemcpyDeviceToHost, h->s_index));
-    FI_CUDA(cudaEventRecord(h->ev_ctr, h->s_index));
-    h->ctr_pending = true;
-  }
-  FI_CUDA(cudaEventRecord(h->ev_index, h->s_index));
-  h->gen_index++;
-  return FI_OK;
-}
-
-// Sharded pools: agree on how many gossip rounds a collective index call needs (the ranks' op counts differ)
-int agree_rounds(fi_epp* h, uint64_t mine, uint64_t* rounds) {
-  *rounds = mine;
-  if (h->world <= 1) return FI_OK;
-  unsigned long long v[2] = {mine, 0};
-  FI_CUDA(cudaMemcpyAsync(h->d_ghdr + 2 * (size_t)h->world, v, sizeof(v), cudaMemcpyHostToDevice, h->s_index));
-  int rc = nccl_allgather_on(h, h->d_ghdr + 2 * (size_t)h->world, h->d_ghdr, sizeof(v), h->s_index);
-  if (rc != FI_OK) return rc;
-  FI_CUDA(cudaMemcpyAsync(h->h_ghdr, h->d_ghdr, (size_t)h->world * sizeof(v), cudaMemcpyDeviceToHost, h->s_index));
-  FI_CUDA(cudaStreamSynchronize(h->s_index));
-  uint64_t m = 0;
-  for (uint32_t g = 0; g < h->world; ++g) m = std::max<uint64_t>(m, h->h_ghdr[2 * g]);
-  *rounds = m;
-  return FI_OK;
-}
-
-// stage one op (already filtered to this shard).  Within a launch group SETs run
-// before CLEARs, so a SET that follows a CLEAR of the same pair starts a new group.
-int submit_op(fi_epp* h, uint64_t hash, uint32_t endpoint, uint32_t op) {
-  if (op == FI_OP_SET) {
-    if (!h->cleared.empty() && h->cleared.count(PairKey{hash, endpoint})) {
-      int rc = flush_ops(h);
-      if (rc != FI_OK) return rc;
-    }
-    h->h_sets[h->cur_buf][h->n_sets++] = fi_index_op{hash, endpoint, FI_OP_SET};
-  } else {
-    h->cleared.insert(PairKey{hash, endpoint});
-    h->h_clears[h->cur_buf][h->n_clears++] = fi_index_op{hash, endpoint, FI_OP_CLEAR};
-  }
-  if (h->n_sets == kOpChunk || h->n_clears == kOpChunk) return flush_ops(h);
-  return FI_OK;
-}
-
-// ---- device-resident LRU (lru_kernels.cu) --------------------------------------------------------------
-// Which LRU serves this handle's indexer.Add calls: decided at the first one.
-int choose_lru_mode(fi_epp* h) {
-  if (h->lru_mode >= 0) return FI_OK;
-  int want = h->lru_want;
-  if (want < 0) {
-    if (const char* e = std::getenv("FI_EPP_DEVICE_LRU")) want = std::strtol(e, nullptr, 10) != 0;
-  }
-  const bool possible = h->cfg.lru_capacity >= h->cfg.max_blocks && h->cfg.lru_capacity <= (1u << 28);
-  if (want == 1 && !possible) return fail(h, FI_ERR_STATE, "device_lru needs lru_capacity >= max_blocks");
-  h->lru_mode = (want < 0 ? possible : want == 1) ? 1 : 0;
-  return FI_OK;
-}
-
-void free_dev_lru(fi_epp* h) {
-  cudaFree(h->dlru.slots);
-  cudaFree(h->dlru.log);
-  cudaFree(h->d_lru_state);
-  cudaFree(h->d_lru_ctr);
-  if (h->h_lru_stat) cudaFreeHost(h->h_lru_stat);
-  cudaFree(h->d_lru_slot_of);
-  cudaFree(h->d_lru_wcount);
-  cudaFree(h->d_lru_base);
-  cudaFree(h->d_lru_sets);
-  cudaFree(h->d_lru_clears);
-  if (h->ev_lru) cudaEventDestroy(h->ev_lru);
-  if (h->ev_lru_ovf) cudaEventDestroy(h->ev_lru_ovf);
-  h->dlru = DevLru{};
-  h->d_lru_state = nullptr;
-  h->d_lru_ctr = nullptr;
-  h->h_lru_stat = nullptr;
-  h->d_lru_slot_of = h->d_lru_wcount = h->d_lru_base = nullptr;
-  h->d_lru_sets = h->d_lru_clears = nullptr;
-  h->ev_lru = h->ev_lru_ovf = nullptr;
-  h->dlru_ready = false;
-}
-
-int alloc_dev_lru(fi_epp* h);
-
-int ensure_dev_lru(fi_epp* h) {
-  if (h->dlru_ready) return FI_OK;
-  const int rc = alloc_dev_lru(h);
-  if (rc != FI_OK) {  // nothing of a partial allocation survives (a later call may succeed, e.g. with the host LRU freed)
-    const std::string why = h->err;
-    cudaGetLastError();
-    free_dev_lru(h);
-    h->err = why;
-    return rc;
-  }
-  h->dlru_ready = true;
-  return FI_OK;
-}
-
-int alloc_dev_lru(fi_epp* h) {
-  const uint32_t EL = h->cfg.endpoint_count, C = h->cfg.lru_capacity;
-  DevLru& d = h->dlru;
-  d.EL = EL;
-  d.capacity = C;
-  size_t free_b = 0, total_b = 0;
-  FI_CUDA(cudaMemGetInfo(&free_b, &total_b));
-  // Log: at least 4 C records (a sub-batch appends at most C; more room = rarer compaction).  Table: at least 4 C slots (C entries + C new keys of a
-  // conservative sub-batch + tombstones); a table takes a batch's DISTINCT keys on top of its entries, and an
-  // endpoint that attracts a popular prefix can receive a large share of a batch — so the tables get as much as
-  // a quarter of the free HBM buys, up to 32 C slots (1 Mi slots = 16 MiB per endpoint at lruCapacityPerServer
-  // 31 250: 17 GB for 1 024 endpoints of a B200's 180).  Option "lru_table_slots" / FI_EPP_LRU_TABLE_SLOTS pins it.
-  d.L = std::max<uint32_t>(pow2_ceil32(4u * C), 64u);
-  const uint32_t ts_min = d.L;
-  uint32_t ts = pow2_ceil32(32u * C);
-  while (ts > ts_min && (size_t)EL * (ts + 2) * sizeof(LruSlot) > free_b / 4) ts >>= 1;
-  uint32_t want = h->lru_table_slots;
-  if (!want)
-    if (const char* ev = std::getenv("FI_EPP_LRU_TABLE_SLOTS")) want = (uint32_t)std::strtoul(ev, nullptr, 10);
-  if (want) ts = std::max(ts_min, pow2_ceil32(want));
-  d.TS = ts;
-  d.L = std::max(d.L, d.TS / 4);
-  d.insert_limit = (uint32_t)((uint64_t)d.TS * 85 / 100);
-  const size_t slot_bytes = (size_t)EL * (d.TS + 2) * sizeof(LruSlot), log_bytes = (size_t)EL * d.L * sizeof(uint64_t);
-  h->lru_touch_cap = std::max<uint64_t>((uint64_t)h->cfg.max_batch * h->MP, 1u << 16);
-  const size_t scratch = (size_t)h->lru_touch_cap * (sizeof(uint32_t) + 3 * sizeof(fi_index_op));
-  if (slot_bytes + log_bytes + scratch + (256u << 20) > free_b)
-    return fail(h, FI_ERR_NOMEM, "device LRU does not fit in free HBM (option device_lru = 0 selects the host LRU)");
-  const size_t state_words = (size_t)7 * EL + 2;
-  FI_CUDA(cudaMalloc(&d.slots, slot_bytes));
-  FI_CUDA(cudaMalloc(&d.log, log_bytes));
-  FI_CUDA(cudaMalloc(&h->d_lru_state, state_words * sizeof(uint32_t)));
-  FI_CUDA(cudaMalloc(&h->d_lru_ctr, 8 * sizeof(unsigned long long)));
-  FI_CUDA(cudaMallocHost(&h->h_lru_stat, sizeof(fi_epp::LruHostStat)));
-  std::memset(h->h_lru_stat, 0, sizeof(fi_epp::LruHostStat));
-  FI_CUDA(cudaMalloc(&h->d_lru_slot_of, h->lru_touch_cap * sizeof(uint32_t)));
-  FI_CUDA(cudaMalloc(&h->d_lru_sets, h->lru_touch_cap * sizeof(fi_index_op)));
-  FI_CUDA(cudaMalloc(&h->d_lru_clears, 2 * h->lru_touch_cap * sizeof(fi_index_op)));  // doomed keys + evictions
-  FI_CUDA(cudaMalloc(&h->d_lru_wcount, (size_t)h->cfg.max_batch * sizeof(uint32_t)));
-  FI_CUDA(cudaMalloc(&h->d_lru_base, (size_t)h->cfg.max_batch * sizeof(uint32_t)));
-  FI_CUDA(cudaEventCreateWithFlags(&h->ev_lru, cudaEventDisableTiming));
-  FI_CUDA(cudaEventCreateWithFlags(&h->ev_lru_ovf, cudaEventDisableTiming));
-  FI_CUDA(cudaMemsetAsync(d.slots, 0, slot_bytes, h->s_index));
-  FI_CUDA(cudaMemsetAsync(h->d_lru_state, 0, state_words * sizeof(uint32_t), h->s_index));
-  FI_CUDA(cudaMemsetAsync(h->d_lru_ctr, 0, 8 * sizeof(unsigned long long), h->s_index));
-  FI_CUDA(cudaEventRecord(h->ev_lru, h->s_index));
-  h->gen_lru++;
-  d.head = h->d_lru_state;
-  d.tail = d.head + EL;
-  d.count = d.tail + EL;
-  d.used = d.count + EL;
-  d.hold = d.used + EL;
-  d.dcount = d.hold + EL;
-  d.ovf = d.dcount + EL;
-  d.any_ovf = d.ovf + EL;
-  d.error = d.any_ovf + 1;
-  d.n_sets = h->d_lru_ctr;
-  d.n_maintained = h->d_lru_ctr + 1;
-  d.n_clears = h->d_lru_ctr + 3;
-  d.n_doomed = h->d_lru_ctr + 4;
-  return FI_OK;
-}
-
-// queue the refresh of the pinned LRU status (error flag + totals) behind everything submitted so far
-int lru_refresh_stat(fi_epp* h) {
-  FI_CUDA(cudaMemcpyAsync(&h->h_lru_stat->error, h->dlru.error, sizeof(uint32_t), cudaMemcpyDeviceToHost, h->s_index));
-  FI_CUDA(cudaMemcpyAsync(&h->h_lru_stat->n_sets, h->d_lru_ctr, 5 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->s_index));
-  return FI_OK;
-}
-
-// indexer.Add(chains[r], endpoints[r]) for r = 0..R-1 through the device LRU.  `chains` is a host pointer
-// (copied to the device first) or, with on_device, memory the index stream can read.  The first pass is
-// OPTIMISTIC: sub-batches are cut only by the scratch arrays' size, and an endpoint whose table cannot take the
-// batch's distinct keys is rolled back and deferred; the deferred requests then run in a second, conservative pass
-// (at most lru_capacity touches per endpoint and sub-batch: always fits).
-int lru_device_add(fi_epp* h, const uint32_t* endpoints, const uint64_t* chains, bool on_device, uint32_t pitch,
-                   const uint32_t* nblocks, uint32_t R, bool conservative = false) {
-  int rc = ensure_dev_lru(h);
-  if (rc != FI_OK) return rc;
-  const uint32_t EL = h->cfg.endpoint_count, lo = h->cfg.endpoint_begin;
-  for (uint32_t r = 0; r < R; ++r)
-    if (nblocks[r] > h->cfg.lru_capacity && endpoints[r] - lo < EL)
-      return fail(h, FI_ERR_INVALID, "device LRU: a chain longer than lru_capacity");
-  rc = flush_ops(h);  // ops staged through fi_epp_index_apply come first
-  if (rc != FI_OK) return rc;
-  rc = check_counters(h);
-  if (rc != FI_OK) return rc;
-  const auto t0 = std::chrono::steady_clock::now();
-  LruPlan& pl = h->lru_plan;
-  // sharded pool: a sub-batch's APPEAR / VANISH transitions must fit the gossip log of one round (at most one SET per
-  // touch; CLEARs: evictions <= keys added, plus doomed entries <= touches)
-  const bool sharded = h->world > 1;
-  const uint64_t cap_touches = sharded ? std::min<uint64_t>(h->lru_touch_cap, kOpChunk / 2) : h->lru_touch_cap;
-  lru_plan_batch(endpoints, nblocks, R, lo, EL, conservative ? h->cfg.lru_capacity : 0xFFFFFFFFu, cap_touches, h->cfg.max_batch, &pl);
-  if (pl.subs.empty() && !sharded) return FI_OK;
-  const size_t K = pl.req_id.size(), nsub = pl.subs.size();
-  // collective on a sharded pool: the ranks' sub-batch counts differ, every one is a gossip round for all
-  uint64_t rounds = nsub;
-  if (sharded) {
-    rc = agree_rounds(h, nsub, &rounds);
-    if (rc != FI_OK) return rc;
-  }
-  const GossipLog glog = gossip_log(h);
-  // staging: req_id | req_ep | req_n | req_off | ep_list | ep_start[nsub][EL+1] | inc[nsub][EL]
-  const size_t words = 5 * K + nsub * ((size_t)2 * EL + 1);
-  FI_CUDA(cudaEventSynchronize(h->ev_lru));  // the previous call's staging (and chain copy) has been consumed
-  if (words > h->lru_plan_cap) {
-    cudaFree(h->d_lru_plan);
-    if (h->h_lru_plan) cudaFreeHost(h->h_lru_plan);
-    h->d_lru_plan = nullptr;
-    h->h_lru_plan = nullptr;
-    h->lru_plan_cap = 0;
-    const size_t cap = words + words / 2 + 1024;
-    FI_CUDA(cudaMalloc(&h->d_lru_plan, cap * sizeof(uint32_t)));
-    FI_CUDA(cudaMallocHost(&h->h_lru_plan, cap * sizeof(uint32_t)));
-    h->lru_plan_cap = cap;
-  }
-  uint32_t* hp = h->h_lru_plan;
-  if (words) {
-  std::memcpy(hp, pl.req_id.data(), K * 4);
-  std::memcpy(hp + K, pl.req_ep.data(), K * 4);
-  std::memcpy(hp + 2 * K, pl.req_n.data(), K * 4);
-  std::memcpy(hp + 3 * K, pl.req_off.data(), K * 4);
-  std::memcpy(hp + 4 * K, pl.ep_list.data(), K * 4);
-  std::memcpy(hp + 5 * K, pl.ep_start.data(), pl.ep_start.size() * 4);
-  std::memcpy(hp + 5 * K + nsub * ((size_t)EL + 1), pl.inc.data(), pl.inc.size() * 4);
-  }
-  // the LRU kernels run on the index stream; like every index update they are ordered behind the picks
-  // submitted so far (a pick sees the index as of its call)
-  FI_CUDA(cudaStreamWaitEvent(h->s_index, h->ev_pick, 0));
-  if (words) FI_CUDA(cudaMemcpyAsync(h->d_lru_plan, hp, words * sizeof(uint32_t), cudaMemcpyHostToDevice, h->s_index));
-  h->stats.h2d_bytes += words * sizeof(uint32_t);
-  const uint64_t* d_chains = chains;
-  if (!on_device && K) {
-    const size_t cw = (size_t)R * pitch;
-    if (cw > h->lru_chains_cap) {
-      cudaFree(h->d_lru_chains);
-      h->d_lru_chains = nullptr;
-      h->lru_chains_cap = 0;
-      FI_CUDA(cudaMalloc(&h->d_lru_chains, cw * sizeof(uint64_t)));
-      h->lru_chains_cap = cw;
-    }
-    // only the rows the plan kept are needed; whole-range copy when most are (one DMA), row copies otherwise
-    if (K * 2 >= R) {
-      FI_CUDA(cudaMemcpyAsync(h->d_lru_chains, chains, cw * sizeof(uint64_t), cudaMemcpyHostToDevice, h->s_index));
-      h->stats.h2d_bytes += cw * sizeof(uint64_t);
-    } else {
-      for (size_t k = 0; k < K; ++k) {
-        const size_t r = pl.req_id[k];
-        FI_CUDA(cudaMemcpyAsync(h->d_lru_chains + r * pitch, chains + r * pitch, (size_t)pl.req_n[k] * sizeof(uint64_t),
-                                cudaMemcpyHostToDevice, h->s_index));
-        h->stats.h2d_bytes += (size_t)pl.req_n[k] * sizeof(uint64_t);
-      }
-    }
-    d_chains = h->d_lru_chains;
-  }
-  const uint32_t* dp = h->d_lru_plan;
-  h->lru_sub_batches += nsub;
-  std::vector<uint8_t> deferred;  // per request of this call: its endpoint overflowed in the optimistic pass
-  std::vector<uint32_t> ovf_host;
-  size_t n_deferred = 0;
-  for (size_t sb = 0; sb < rounds; ++sb) {
-    if (sb >= nsub) {  // (sharded) this rank is done: it only takes part in the others' gossip rounds
-      rc = gossip_round(h);
-      if (rc != FI_OK) return rc;
-      continue;
-    }
-    if (sb) {  // the index counters of the previous sub-batch decide about a rebuild before more keys arrive
-      rc = check_counters(h);
-      if (rc != FI_OK) return rc;
-    }
-    const LruSubBatch& sbt = pl.subs[sb];
-    LruBatch b{};
-    b.req_id = dp + sbt.k_begin;
-    b.req_ep = dp + K + sbt.k_begin;
-    b.req_n = dp + 2 * K + sbt.k_begin;
-    b.req_off = dp + 3 * K + sbt.k_begin;
-    b.ep_list = dp + 4 * K + sbt.k_begin;
-    b.ep_start = dp + 5 * K + sb * ((size_t)EL + 1);
-    const uint32_t* inc = dp + 5 * K + nsub * ((size_t)EL + 1) + sb * (size_t)EL;
-    b.chains = d_chains;
-    b.pitch = pitch;
-    b.K = sbt.k_end - sbt.k_begin;
-    b.slot_of = h->d_lru_slot_of;
-    b.wcount = h->d_lru_wcount;
-    b.base = h->d_lru_base;
-    b.sets = h->d_lru_sets;
-    {
-      LaunchScope ls(h, h->s_index, K_INDEX);
-      FI_CUDA(launch_lru_maintain(h->dlru, inc, false, h->s_index));
-    }
-    {
-      LaunchScope ls(h, h->s_index, K_INDEX);
-      FI_CUDA(launch_lru_touch(h->dlru, b, h->s_index));
-    }
-    // did some endpoint's table refuse keys?  (one host round trip per sub-batch; everything after it is queued
-    // without waiting)
-    FI_CUDA(cudaMemcpyAsync(&h->h_lru_stat->any_ovf, h->dlru.any_ovf, sizeof(uint32_t), cudaMemcpyDeviceToHost, h->s_index));
-    FI_CUDA(cudaEventRecord(h->ev_lru_ovf, h->s_index));
-    FI_CUDA(cudaEventSynchronize(h->ev_lru_ovf));
-    const bool any_ovf = h->h_lru_stat->any_ovf != 0;
-    if (any_ovf) {
-      if (conservative) return fail(h, FI_ERR_STATE, "device LRU: overflow in a conservative sub-batch");
-      {
-        LaunchScope ls(h, h->s_index, K_INDEX);
-        FI_CUDA(launch_lru_untouch(h->dlru, b, h->s_index));
-      }
-      ovf_host.resize(EL);
-      FI_CUDA(cudaMemcpyAsync(ovf_host.data(), h->dlru.ovf, (size_t)EL * sizeof(uint32_t), cudaMemcpyDeviceToHost, h->s_index));
-      FI_CUDA(cudaStreamSynchronize(h->s_index));
-      if (deferred.empty()) deferred.assign(R, 0);
-      for (uint32_t k = sbt.k_begin; k < sbt.k_end; ++k)
-        if (ovf_host[pl.req_ep[k]]) {
-          deferred[pl.req_id[k]] = 1;
-          ++n_deferred;
-        }
-    }
-    FI_CUDA(cudaMemsetAsync(h->d_lru_ctr + 2, 0, sizeof(unsigned long long), h->s_index));
-    {
-      LaunchScope ls(h, h->s_index, K_INDEX);
-      FI_CUDA(launch_lru_count(h->dlru, b, h->s_index));
-    }
-    {
-      LaunchScope ls(h, h->s_index, K_INDEX);
-      FI_CUDA(launch_lru_scan(h->dlru, b, h->s_index));
-    }
-    {
-      LaunchScope ls(h, h->s_index, K_INDEX);
-      FI_CUDA(launch_lru_append(h->dlru, b, h->d_lru_clears, h->d_lru_ctr + 2, 2 * h->lru_touch_cap, lo, h->s_index));
-    }
-    {
-      LaunchScope ls(h, h->s_index, K_INDEX);
-      FI_CUDA(launch_index_set(h->ix, h->d_ctr, h->d_lru_sets, sbt.touches, lo, EL, h->rank, glog, h->s_index));
-    }
-    {
-      LaunchScope ls(h, h->s_index, K_INDEX);
-      FI_CUDA(launch_lru_evict(h->dlru, h->d_lru_clears, h->d_lru_ctr + 2, 2 * h->lru_touch_cap, lo, h->s_index));
-    }
-    {
-      // CLEARs of a sub-batch: at most one per doomed key (<= touches) and one per eviction (<= keys it added)
-      const uint64_t cap = std::min<uint64_t>(2 * h->lru_touch_cap, 2 * sbt.touches);
-      LaunchScope ls(h, h->s_index, K_INDEX);
-      FI_CUDA(launch_index_clear_counted(h->ix, h->d_ctr, h->d_lru_clears, cap, h->d_lru_ctr + 2, lo, EL, h->rank, glog,
-                                         h->s_index));
-    }
-    if (any_ovf) FI_CUDA(cudaMemsetAsync(h->dlru.ovf, 0, ((size_t)EL + 1) * sizeof(uint32_t), h->s_index));  // ovf[] and any_ovf
-    FI_CUDA(cudaMemcpyAsync(h->h_ctr, h->d_ctr, sizeof(IndexCounters), cudaMemcpyDeviceToHost, h->s_index));
-    FI_CUDA(cudaEventRecord(h->ev_ctr, h->s_index));
-    h->ctr_pending = true;
-    if (sharded) {  // the other ranks replay this sub-batch's transitions into their directories (and we theirs)
-      rc = gossip_round(h);
-      if (rc != FI_OK) return rc;
-    }
-  }
-  rc = lru_refresh_stat(h);
-  if (rc != FI_OK) return rc;
-  FI_CUDA(cudaEventRecord(h->ev_ctr, h->s_index));  // covers the status copy too
-  FI_CUDA(cudaEventRecord(h->ev_lru, h->s_index));
-  h->gen_lru++;
-  FI_CUDA(cudaEventRecord(h->ev_index, h->s_index));
-  h->gen_index++;
-  if (h->verbose) {
-    const auto t1 = std::chrono::steady_clock::now();
-    std::fprintf(stderr, "[fi_epp] device LRU%s: %u requests (%zu kept), %zu sub-batch(es), %zu deferred, host side %.3f ms\n",
-                 conservative ? " (conservative pass)" : "", R, K, nsub, n_deferred,
-                 std::chrono::duration<double, std::milli>(t1 - t0).count());
-  }
-  h->lru_deferred += n_deferred;
-  if (n_deferred || (sharded && !conservative)) {  // (sharded: every rank enters the second pass, most with nothing to do)
-    std::vector<uint32_t> ep2(R);
-    for (uint32_t r = 0; r < R; ++r) ep2[r] = (n_deferred && deferred[r]) ? endpoints[r] : FI_NO_ENDPOINT;
-    return lru_device_add(h, ep2.data(), d_chains, true, pitch, nblocks, R, true);
-  }
-  return FI_OK;
-}
-
-int upload_endpoints(fi_epp* h) {
-  if (!h->eps_dirty) return FI_OK;
-  FI_CUDA(cudaMemcpyAsync(h->d_eps, h->eps.data(), h->eps.size() * sizeof(EndpointDev), cudaMemcpyHostToDevice, h->s_main));
-  h->stats.h2d_bytes += h->eps.size() * sizeof(EndpointDev);
-  {
-    LaunchScope ls(h, h->s_main, K_OTHER);
-    FI_CUDA(launch_prepare_endpoints(h->d_eps, h->cfg.num_endpoints, h->cfg.endpoint_begin, h->cfg.endpoint_count, h->st,
-                                     h->d_sc, h->d_elig, h->d_zero, h->d_ztie, h->s_main));
-  }
-  // eps is pageable host memory: the copy above has been staged by the time the call returns
-  h->eps_dirty = false;
-  return FI_OK;
-}
-
-int upload_lora(fi_epp* h) {
-  if (!h->lora_dirty) return FI_OK;
-  FI_CUDA(cudaMemcpyAsync(h->d_lora, h->lora.data(), h->lora.size() * sizeof(LoraDev), cudaMemcpyHostToDevice, h->s_main));
-  h->stats.h2d_bytes += h->lora.size() * sizeof(LoraDev);
-  h->lora_dirty = false;
-  return FI_OK;
-}
-
-// hash kernels for the request slice [r0, r0+R): prompts → chain (device buffers), on stream s
-int run_hash(fi_epp* h, const uint8_t* d_prompts, const uint64_t* d_offsets, const uint64_t* d_h0, uint32_t r0,
-             uint32_t R, cudaStream_t s) {
-  uint64_t* pre = h->d_pre + (size_t)r0 * h->MP;  // tiled by groups of 32 requests: r0 % 32 == 0
-  uint64_t* chain = h->d_chain + (size_t)r0 * h->MP;
-  uint32_t* nb = h->d_nblocks + r0;
-  if (h->fast_hash) {
-    {
-      LaunchScope ls(h, s, K_HASH);
-      FI_CUDA(launch_hash_blocks(d_prompts, d_offsets + r0, R, h->cfg.block_bytes, h->cfg.max_blocks, h->MP, pre, nb, 0, s));
-    }
-    LaunchScope ls(h, s, K_CHAIN);
-    FI_CUDA(launch_chain_finalize(pre, nb, d_h0 + r0, R, h->MP, chain, false, s));
-  } else {
-    LaunchScope ls(h, s, K_HASH);
-    FI_CUDA(launch_hash_generic(d_prompts, d_offsets + r0, d_h0 + r0, R, h->cfg.block_bytes, h->cfg.max_blocks, h->MP,
-                                chain, nb, s));
-  }
-  return FI_OK;
-}
-
-int nccl_allgather_on(fi_epp* h, const void* send, void* recv, size_t bytes, cudaStream_t s) {
-  int rc = g_nccl.AllGather(send, recv, bytes, ncclInt8, h->comm, s);
-  if (rc != ncclSuccess)
-    return fail(h, FI_ERR_COMM, std::string("ncclAllGather: ") + (g_nccl.GetErrorString ? g_nccl.GetErrorString(rc) : "error"));
-  return FI_OK;
-}
-int nccl_allgather(fi_epp* h, const void* send, void* recv, size_t bytes) { return nccl_allgather_on(h, send, recv, bytes, h->s_main); }
-
-// Peer-memory exchange set-up (sharded mode): allocate this rank's buffer, exchange its IPC handle over
-// the NCCL communicator, map every peer's buffer.  Falls back to the NCCL all-gather path (px.enabled = 0)
-// when FI_EPP_EXCHANGE=nccl, when there are more than FI_MAX_RANKS ranks, or when any rank cannot map a peer.
-struct XchgBlob {
-  cudaIpcMemHandle_t handle;
-  uint64_t ptr;
-  int64_t pid;
-  int32_t device;
-  int32_t ok;
-  uint8_t pad[40];
-};
-static_assert(sizeof(XchgBlob) == 128, "XchgBlob size");
-
-int setup_peer_exchange(fi_epp* h) {
-  const char* mode = std::getenv("FI_EPP_EXCHANGE");
-  const bool want = !(mode && std::strcmp(mode, "nccl") == 0) && h->world <= (uint32_t)FI_MAX_RANKS;
-  const uint64_t R = h->cfg.max_batch;
-  auto up = [](uint64_t v) { return (v + 255) & ~255ull; };
-  PeerXchg px{};
-  px.world = h->world;
-  px.rank = h->rank;
-  uint64_t off = 0;
-  for (int par = 0; par < 2; ++par) {  // tagged 64-bit words (kernels.cuh PeerXchg)
-    px.off_pick[par] = off;
-    off = up(off + (uint64_t)h->world * R * h->P * 4 * sizeof(uint64_t));
-  }
-  XchgBlob mine{};
-  mine.ok = 0;
-  if (want && cudaMalloc(&h->d_xchg, off) == cudaSuccess && cudaMemset(h->d_xchg, 0, off) == cudaSuccess &&
-      cudaHostAlloc((void**)&h->h_xerr, sizeof(uint32_t), cudaHostAllocMapped) == cudaSuccess &&
-      cudaIpcGetMemHandle(&mine.handle, h->d_xchg) == cudaSuccess) {
-    mine.ok = 1;
-  }
-  cudaGetLastError();
-  mine.ptr = (uint64_t)(uintptr_t)h->d_xchg;
-  mine.pid = (int64_t)getpid();
-  mine.device = h->cfg.device;
-  // round 1: handles; round 2: "I mapped every peer" votes.  Both ride the NCCL communicator.
-  XchgBlob* d_blobs = nullptr;
-  FI_CUDA(cudaMalloc(&d_blobs, (size_t)(h->world + 1) * sizeof(XchgBlob)));
-  std::vector<XchgBlob> all(h->world);
-  auto gather = [&]() -> int {
-    FI_CUDA(cudaMemcpyAsync(d_blobs + h->world, &mine, sizeof(mine), cudaMemcpyHostToDevice, h->s_main));
-    int rc = nccl_allgather(h, d_blobs + h->world, d_blobs, sizeof(XchgBlob));
-    if (rc != FI_OK) return rc;
-    FI_CUDA(cudaMemcpyAsync(all.data(), d_blobs, (size_t)h->world * sizeof(XchgBlob), cudaMemcpyDeviceToHost, h->s_main));
-    FI_CUDA(cudaStreamSynchronize(h->s_main));
-    return FI_OK;
-  };
-  int rc = gather();
-  if (rc != FI_OK) {
-    cudaFree(d_blobs);
-    return rc;
-  }
-  bool ok = true;
-  for (uint32_t k = 0; k < h->world; ++k) ok = ok && all[k].ok;
-  if (ok) {
-    for (uint32_t k = 0; k < h->world && ok; ++k) {
-      if (k == h->rank) {
-        px.base[k] = h->d_xchg;
-      } else if (all[k].pid == mine.pid) {  // same process: plain peer access
-        int can = 0;
-        if (all[k].device != h->cfg.device) {
-          cudaDeviceCanAccessPeer(&can, h->cfg.device, all[k].device);
-          if (can) {
-            cudaError_t e = cudaDeviceEnablePeerAccess(all[k].device, 0);
-            can = (e == cudaSuccess || e == cudaErrorPeerAccessAlreadyEnabled);
-            cudaGetLastError();
-          }
-        } else {
-          can = 1;
-        }
-        ok = can != 0;
-        px.base[k] = (uint8_t*)(uintptr_t)all[k].ptr;
-      } else {
-        void* m = nullptr;
-        if (cudaIpcOpenMemHandle(&m, all[k].handle, cudaIpcMemLazyEnablePeerAccess) == cudaSuccess) {
-          h->peer_ipc[k] = m;
-          px.base[k] = (uint8_t*)m;
-        } else {
-          cudaGetLastError();
-          ok = false;
-        }
-      }
-    }
-  }
-  mine.ok = ok ? 1 : 0;
-  rc = gather();
-  cudaFree(d_blobs);
-  if (rc != FI_OK) return rc;
-  for (uint32_t k = 0; k < h->world; ++k) ok = ok && all[k].ok;
-  if (ok) {
-    px.enabled = 1;
-    px.step = 0;
-    *h->h_xerr = 0;
-    px.err = const_cast<uint32_t*>(h->h_xerr);  // unified addressing: the host pointer is the device pointer
-  }
-  h->px = px;
-  if (std::getenv("FI_EPP_VERBOSE"))
-    std::fprintf(stderr, "[fi_epp] rank %u/%u: sharded exchange over %s\n", h->rank, h->world,
-                 px.enabled ? "peer memory (in-kernel tagged stores)" : "NCCL all-gather");
-  return FI_OK;
-}
-
-// FI_EPP_TRACE=<call index>: print that call's kernel timeline (start/end relative to the call's start)
-void dump_trace(fi_epp* h, uint32_t R) {
-  if (!h->tracing) return;
-  static const char* names[] = {"hash_blocks", "chain_finalize", "match_pick", "index", "other"};
-  cudaStreamSynchronize(h->s_main);
-  std::fprintf(stderr, "[fi_epp trace] rank %u call %ld: R=%u\n", h->rank, h->trace_call, R);
-  for (auto& e : h->pending_ev) {
-    float t0 = 0.f, t1 = 0.f;
-    cudaEventSynchronize(e.b);
-    cudaEventElapsedTime(&t0, h->ev_trace0, e.a);
-    cudaEventElapsedTime(&t1, h->ev_trace0, e.b);
-    std::fprintf(stderr, "[fi_epp trace]   r%u %-15s start %8.1f us  end %8.1f us  (%6.1f us)\n", h->rank, names[e.kind],
-                 t0 * 1e3, t1 * 1e3, (t1 - t0) * 1e3);
-    h->ev_pool.push_back(e.a);
-    h->ev_pool.push_back(e.b);
-  }
-  h->pending_ev.clear();
-  h->tracing = false;
-}
-
-// host prompts still to be copied (fi_epp_pick_batch): run_pick copies them, in slices when it can
-struct HostFeed {
-  const uint8_t* prompts;   // host
-  const uint64_t* offsets;  // host, [R+1]
-};
-
-void fill_match_params(fi_epp* h, MatchParams& mp, const uint64_t* chain, const uint32_t* nb, const uint64_t* d_offsets,
-                       const uint64_t* d_h0, const uint64_t* d_adapters, uint32_t R, fi_pick* out, bool local_pd) {
-  mp.chain = chain;
-  mp.nblocks = nb;
-  mp.offsets = d_offsets;
-  mp.adapters = d_adapters;
-  mp.R = R;
-  mp.MP = h->MP;
-  mp.ix = h->ix;
-  mp.st = h->st;
-  mp.ep_begin = h->cfg.endpoint_begin;
-  mp.ep_count = h->cfg.endpoint_count;
-  mp.E_global = h->cfg.num_endpoints;
-  mp.r_base = 0;
-  mp.h0 = d_h0;
-  mp.lpm = h->cfg.match_mode;
-  mp.apply_pd = (h->cfg.pd_enabled && local_pd) ? 1 : 0;
-  mp.pd_decode = h->cfg.pd_decode_profile;
-  mp.pd_prefill = h->cfg.pd_prefill_profile;
-  mp.pd_threshold = h->cfg.pd_threshold;
-  mp.out = out;
-  mp.probed_blocks = h->profiling ? h->d_probed : nullptr;
-  mp.work_counter = h->d_work;
-  mp.zero_work_counter = 1;
-  mp.lane_zero = 0;
-}
-
-// the whole pick on device buffers; result in d_out ([R][P])
-int run_pick_impl(fi_epp* h, const uint8_t* d_prompts, const uint64_t* d_offsets, const uint64_t* d_h0,
-                  const uint64_t* d_adapters, uint32_t R, fi_pick* d_out, const HostFeed* feed) {
-  const bool sharded = h->world > 1;
-  if (sharded && (h->n_sets || h->n_clears))
-    return fail(h, FI_ERR_STATE, "sharded pool: index updates are collective (fi_epp_index_apply / fi_epp_index_add_chains)");
-  int rc = flush_ops(h);
-  if (rc != FI_OK) return rc;
-  rc = check_counters(h);
-  if (rc != FI_OK) return rc;
-  h->tracing = !h->profiling && h->trace_call >= 0 && (long)h->stats.pick_calls == h->trace_call;
-  if (h->tracing) {
-    if (!h->ev_trace0) cudaEventCreate(&h->ev_trace0);
-    FI_CUDA(cudaStreamSynchronize(h->s_main));
-    FI_CUDA(cudaEventRecord(h->ev_trace0, h->s_main));
-  }
-  FI_CUDA(cudaStreamWaitEvent(h->s_main, h->ev_index, 0));  // every submitted op is visible
-  rc = upload_endpoints(h);
-  if (rc != FI_OK) return rc;
-  rc = upload_lora(h);
-  if (rc != FI_OK) return rc;
-  if (h->pipe_seq) {  // a plain pick after pipelined submits: their stages share d_pre / d_chain with ours
-    FI_CUDA(cudaStreamWaitEvent(h->s_main, h->ev_a[(h->pipe_seq - 1) & 1], 0));
-    FI_CUDA(cudaStreamWaitEvent(h->s_main, h->ev_pick, 0));  // (their matches may run on the partition's stream)
-    h->part_active = false;
-  }
-  MatchParams mp{};
-  fill_match_params(h, mp, h->d_chain, h->d_nblocks, d_offsets, d_h0, d_adapters, R, sharded ? h->d_local : d_out, !sharded);
-
-  const uint32_t S = h->feed_slices;
-  if (feed && !sharded && h->fast_hash && S > 1 && R >= 64 * S && feed->offsets[R] >= (8ull << 20)) {
-    // Sliced feed.  (On DEVICE-resident inputs slicing the step is slower — DESIGN.md "What did not
-    // work" — but here the copy engine is the bottleneck and the kernels of slice k hide under copy k+1.)
-    uint8_t* dp = const_cast<uint8_t*>(d_prompts);
-    const uint32_t per = (((R + S - 1) / S) + 31) & ~31u;
-    uint32_t used = 0;
-    for (uint32_t k = 0; k * per < R; ++k, ++used) {
-      const uint32_t r0 = k * per, r1 = std::min(R, r0 + per);
-      const uint64_t b0 = feed->offsets[r0], b1 = feed->offsets[r1];
-      if (b1 > b0) FI_CUDA(cudaMemcpyAsync(dp + b0, feed->prompts + b0, b1 - b0, cudaMemcpyHostToDevice, h->s_copy));
-      FI_CUDA(cudaEventRecord(h->ev_copy[k], h->s_copy));
-    }
-    h->stats.h2d_bytes += feed->offsets[R];
-    for (uint32_t k = 0; k < used; ++k) {
-      const uint32_t r0 = k * per, Rk = std::min(per, R - r0);
-      FI_CUDA(cudaStreamWaitEvent(h->s_main, h->ev_copy[k], 0));
-      rc = run_hash(h, d_prompts, d_offsets, d_h0, r0, Rk, h->s_main);
-      if (rc != FI_OK) return rc;
-      MatchParams ms = mp;
-      ms.chain = mp.chain + (size_t)r0 * h->MP;
-      ms.nblocks = mp.nblocks + r0;
-      ms.offsets = mp.offsets ? mp.offsets + r0 : nullptr;
-      ms.adapters = mp.adapters ? mp.adapters + r0 : nullptr;
-      ms.h0 = mp.h0 + r0;
-      ms.r_base = r0;
-      ms.R = Rk;
-      ms.out = mp.out + (size_t)r0 * h->P;
-      ms.work_counter = h->d_work + k;
-      LaunchScope ls(h, h->s_main, K_MATCH);
-      FI_CUDA(launch_match_pick(ms, h->sm_count, h->s_main));
-    }
-    dump_trace(h, R);
-    h->stats.pick_calls++;
-    h->stats.requests += R;
-    return FI_OK;
-  }
-  if (feed && feed->offsets[R]) {  // one copy, then the whole batch
-    FI_CUDA(cudaMemcpyAsync(const_cast<uint8_t*>(d_prompts), feed->prompts, feed->offsets[R], cudaMemcpyHostToDevice, h->s_main));
-    h->stats.h2d_bytes += feed->offsets[R];
-  }
-  if (!sharded) {
-    // (A sub-batch pipeline over several streams was tried and measured slower on device-resident
-    // inputs — DESIGN.md "What did not work": the chain walk costs a flat serial latency at any batch
-    // size and small slices pay launch/ramp overheads.)
-    rc = run_hash(h, d_prompts, d_offsets, d_h0, 0, R, h->s_main);
-    if (rc != FI_OK) return rc;
-    {
-      LaunchScope ls(h, h->s_main, K_MATCH);
-      FI_CUDA(launch_match_pick(mp, h->sm_count, h->s_main));
-    }
-    dump_trace(h, R);
-    h->stats.pick_calls++;
-    h->stats.requests += R;
-    return FI_OK;
-  }
-
-  // ---- endpoint-range sharded pool --------------------------------------------------------------
-  // Hashing: every rank needs every request's chain.  split: rank g hashes requests [g·per, (g+1)·per) and
-  // the chain rows + block counts are all-gathered in place (2 KiB per request over NVLink instead of
-  // re-reading 16 KiB of prompt on every rank); replicated: every rank hashes everything.
-  if (h->split_hash && h->fast_hash && R >= 32 * h->world) {
-    const uint32_t per = (((R + h->world - 1) / h->world) + 31) & ~31u;  // ≤ chain_rows / world
-    const uint32_t r0 = std::min(R, h->rank * per), r1 = std::min(R, r0 + per);
-    if (r1 > r0) {
-      rc = run_hash(h, d_prompts, d_offsets, d_h0, r0, r1 - r0, h->s_main);
-      if (rc != FI_OK) return rc;
-    }
-    rc = nccl_allgather(h, h->d_chain + (size_t)h->rank * per * h->MP, h->d_chain, (size_t)per * h->MP * sizeof(uint64_t));
-    if (rc != FI_OK) return rc;
-    rc = nccl_allgather(h, h->d_nblocks + (size_t)h->rank * per, h->d_nblocks, (size_t)per * sizeof(uint32_t));
-    if (rc != FI_OK) return rc;
-    h->stats.n_other += 2;  // two collectives of the step (not kernels of this library)
-  } else {
-    rc = run_hash(h, d_prompts, d_offsets, d_h0, 0, R, h->s_main);
-    if (rc != FI_OK) return rc;
-  }
-  const bool p2p = h->px.enabled != 0;
-  if (p2p) {
-    // Peer-memory exchange: match_pick stores this rank's picks as tagged words into every rank's buffer and
-    // merge_picks polls per request, so the reduction has no collective call, no barrier between the ranks
-    // and no host round trip.  A timeout is reported once (the kernels set the mapped host word).
-    if (*h->h_xerr) {
-      *h->h_xerr = 0;
-      return fail(h, FI_ERR_COMM, "peer exchange timed out waiting for another rank");
-    }
-    h->px.step += 1;
-    if (h->px.step == 0) h->px.step = 1;  // tag 0 is the zero-initialised buffer
-    mp.px = h->px;
-  }
-  {
-    LaunchScope ls(h, h->s_main, K_MATCH);
-    FI_CUDA(launch_match_pick(mp, h->sm_count, h->s_main));
-  }
-  MergeParams mg{};
-  if (p2p) {
-    mg.gathered = reinterpret_cast<const fi_pick*>(h->d_xchg + h->px.off_pick[h->px.step & 1u]);
-    mg.px = h->px;
-  } else {
-    rc = nccl_allgather(h, h->d_local, h->d_gather, (size_t)R * h->P * sizeof(fi_pick));
-    if (rc != FI_OK) return rc;
-    mg.gathered = h->d_gather;
-  }
-  mg.ranks = h->world;
-  mg.R = R;
-  mg.P = h->P;
-  mg.nblocks = h->d_nblocks;
-  mg.offsets = d_offsets;
-  mg.chain = h->d_chain;
-  mg.h0 = d_h0;
-  mg.MP = h->MP;
-  mg.E_global = h->cfg.num_endpoints;
-  mg.apply_pd = h->cfg.pd_enabled;
-  mg.pd_decode = h->cfg.pd_decode_profile;
-  mg.pd_prefill = h->cfg.pd_prefill_profile;
-  mg.pd_threshold = h->cfg.pd_threshold;
-  mg.out = d_out;
-  {
-    LaunchScope ls(h, h->s_main, K_OTHER);
-    FI_CUDA(launch_merge_picks(mg, h->s_main));
-  }
-  dump_trace(h, R);
-  h->stats.pick_calls++;
-  h->stats.requests += R;
-  return FI_OK;
-}
-
-int run_pick(fi_epp* h, const uint8_t* d_prompts, const uint64_t* d_offsets, const uint64_t* d_h0,
-             const uint64_t* d_adapters, uint32_t R, fi_pick* d_out, const HostFeed* feed = nullptr) {
-  int rc = run_pick_impl(h, d_prompts, d_offsets, d_h0, d_adapters, R, d_out, feed);
-  if (rc != FI_OK) return rc;
-  h->ev_pick = h->ev_pick_own;
-  FI_CUDA(cudaEventRecord(h->ev_pick, h->s_main));  // index updates submitted later wait for this pick
-  FI_CUDA(cudaEventRecord(h->ev_plain, h->s_main));
-  h->gen_plain++;
-  h->last_plain_R = R;
-  return FI_OK;
-}
-
-// ---- SM partition of the pipelined path (green contexts through the driver entry points) ------------------
-struct GreenApi {
-  CUresult (*DeviceGet)(CUdevice*, int) = nullptr;
-  CUresult (*DeviceGetDevResource)(CUdevice, CUdevResource*, CUdevResourceType) = nullptr;
-  CUresult (*DevSmResourceSplitByCount)(CUdevResource*, unsigned int*, const CUdevResource*, CUdevResource*, unsigned int,
-                                        unsigned int) = nullptr;
-  CUresult (*DevResourceGenerateDesc)(CUdevResourceDesc*, CUdevResource*, unsigned int) = nullptr;
-  CUresult (*GreenCtxCreate)(CUgreenCtx*, CUdevResourceDesc, CUdevice, unsigned int) = nullptr;
-  CUresult (*GreenCtxDestroy)(CUgreenCtx) = nullptr;
-  CUresult (*GreenCtxStreamCreate)(CUstream*, CUgreenCtx, unsigned int, int) = nullptr;
-  bool loaded = false, ok = false;
-};
-GreenApi g_green;
-
-bool load_green_api() {
-  if (g_green.loaded) return g_green.ok;
-  g_green.loaded = true;
-  auto get = [](const char* name, void** fn) {
-    cudaDriverEntryPointQueryResult qr;
-    return cudaGetDriverEntryPoint(name, fn, cudaEnableDefault, &qr) == cudaSuccess && qr == cudaDriverEntryPointSuccess && *fn;
-  };
-  g_green.ok = get("cuDeviceGet", (void**)&g_green.DeviceGet) &&
-               get("cuDeviceGetDevResource", (void**)&g_green.DeviceGetDevResource) &&
-               get("cuDevSmResourceSplitByCount", (void**)&g_green.DevSmResourceSplitByCount) &&
-               get("cuDevResourceGenerateDesc", (void**)&g_green.DevResourceGenerateDesc) &&
-               get("cuGreenCtxCreate", (void**)&g_green.GreenCtxCreate) &&
-               get("cuGreenCtxDestroy", (void**)&g_green.GreenCtxDestroy) &&
-               get("cuGreenCtxStreamCreate", (void**)&g_green.GreenCtxStreamCreate);
-  cudaGetLastError();
-  return g_green.ok;
-}
-
-void destroy_partition(fi_epp* h) {
-  if (g_green.ok) {
-    if (h->gctx_walk) g_green.GreenCtxDestroy(h->gctx_walk);
-    if (h->gctx_main) g_green.GreenCtxDestroy(h->gctx_main);
-  }
-  h->gctx_walk = h->gctx_main = nullptr;
-}
-
-// Try to split the GPU; on any failure the pipelined path keeps running unpartitioned.
-void setup_partition(fi_epp* h) {
-  if (h->part_state != 0) return;
-  h->part_state = -1;
-  if (h->part_want <= 0 || h->world > 1 || !load_green_api()) return;
-  CUdevice dev;
-  CUdevResource all{}, grp{}, rem{};
-  unsigned int nb = 1;
-  if (g_green.DeviceGet(&dev, h->cfg.device) != CUDA_SUCCESS) return;
-  if (g_green.DeviceGetDevResource(dev, &all, CU_DEV_RESOURCE_TYPE_SM) != CUDA_SUCCESS) return;
-  if (g_green.DevSmResourceSplitByCount(&grp, &nb, &all, &rem, 0, (unsigned)h->part_want) != CUDA_SUCCESS || nb != 1) return;
-  if (grp.sm.smCount < 8 || rem.sm.smCount < 64) return;
-  CUdevResourceDesc dw = nullptr, dm = nullptr;
-  if (g_green.DevResourceGenerateDesc(&dw, &grp, 1) != CUDA_SUCCESS) return;
-  if (g_green.DevResourceGenerateDesc(&dm, &rem, 1) != CUDA_SUCCESS) return;
-  if (g_green.GreenCtxCreate(&h->gctx_walk, dw, dev, CU_GREEN_CTX_DEFAULT_STREAM) != CUDA_SUCCESS) return;
-  if (g_green.GreenCtxCreate(&h->gctx_main, dm, dev, CU_GREEN_CTX_DEFAULT_STREAM) != CUDA_SUCCESS) {
-    destroy_partition(h);
-    return;
-  }
-  // hash_blocks(k+2) and match_pick(k) become runnable at the same moment (both wait for match_pick(k-1)) and share
-  // the big partition; which of them gets its CTAs resident first decided the step — 116 us on some boxes, 138 us
-  // on others with the same code.  Stream priorities make the block scheduler prefer one of them whenever SMs free
-  // up (FI_EPP_PIPE_PRIO=match | hash | none).
-  int prio_lo = 0, prio_hi = 0;
-  cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi);  // lo = least (numerically greatest), hi = greatest priority
-  int pa = 0, pb = 0;
-  const char* pe = std::getenv("FI_EPP_PIPE_PRIO");
-  const std::string prio = pe ? pe : "none";  // (measured on a 116-us box: none 116.1, hash 116.2, match 121.2 us)
-  if (prio == "match") {
-    pa = prio_lo;
-    pb = prio_hi;
-  } else if (prio == "hash") {
-    pa = prio_hi;
-    pb = prio_lo;
-  }
-  CUstream sw = nullptr, sa = nullptr, sb = nullptr;
-  if (g_green.GreenCtxStreamCreate(&sw, h->gctx_walk, CU_STREAM_NON_BLOCKING, 0) != CUDA_SUCCESS ||
-      g_green.GreenCtxStreamCreate(&sa, h->gctx_main, CU_STREAM_NON_BLOCKING, pa) != CUDA_SUCCESS ||
-      g_green.GreenCtxStreamCreate(&sb, h->gctx_main, CU_STREAM_NON_BLOCKING, pb) != CUDA_SUCCESS) {
-    destroy_partition(h);
-    return;
-  }
-  h->s_pw = (cudaStream_t)sw;
-  h->s_pa = (cudaStream_t)sa;
-  h->s_pb = (cudaStream_t)sb;
-  bool ok = cudaMalloc(&h->d_pre2, (size_t)h->chain_rows * h->MP * sizeof(uint64_t)) == cudaSuccess &&
-            cudaMalloc(&h->d_nblocks3, (size_t)h->cfg.max_batch * sizeof(uint32_t)) == cudaSuccess;
-  for (cudaEvent_t* e : {&h->ev_h[0], &h->ev_h[1], &h->ev_b3[0], &h->ev_b3[1], &h->ev_b3[2], &h->ev_up})
-    ok = ok && cudaEventCreateWithFlags(e, cudaEventDisableTiming) == cudaSuccess;
-  if (!ok) {
-    cudaGetLastError();
-    return;
-  }
-  h->part_walk_sms = (int)grp.sm.smCount;
-  h->part_main_sms = (int)rem.sm.smCount;
-  h->part_state = 1;
-  if (h->verbose)
-    std::fprintf(stderr, "[fi_epp] pipelined path: SM partition %d (chain walk) + %d (hashing, matching), three batches in flight\n",
-                 h->part_walk_sms, h->part_main_sms);
-}
-
-// Pipelined device path on the partitioned GPU: hash(k) and match(k) on the big partition's two streams,
-// chain(k) on the walker partition.  Buffers: pre[2] and chain[2] by batch parity, nblocks[3] by k mod 3 (hash(k+2)
-// writes its block counts while match(k) still reads its own).
-int submit_pick_partitioned(fi_epp* h, const uint8_t* d_prompts, const uint64_t* d_offsets, const uint64_t* d_h0, uint32_t R,
-                            fi_pick* d_out, cudaStream_t us) {
-  const uint64_t k = h->pipe_seq;
-  const uint32_t s2 = (uint32_t)(k & 1), s3 = (uint32_t)(k % 3);
-  uint64_t* pre = s2 ? h->d_pre2 : h->d_pre;
-  uint64_t* chain = s2 ? h->d_chain2 : h->d_chain;
-  uint32_t* nb = s3 == 0 ? h->d_nblocks : (s3 == 1 ? h->d_nblocks2 : h->d_nblocks3);
-  // ---- hash(k): inputs ready in the caller's stream order; pre[s2] free once chain(k-2) has read it, nb[s3] once
-  // match(k-3) has; d_pre / d_chain are shared with stream-ordered picks and with the device LRU's reads
-  FI_CUDA(cudaEventRecord(h->ev_in, us));
-  FI_CUDA(cudaStreamWaitEvent(h->s_pa, h->ev_in, 0));
-  if (h->seen_plain != h->gen_plain) {
-    FI_CUDA(cudaStreamWaitEvent(h->s_pa, h->ev_plain, 0));
-    h->seen_plain = h->gen_plain;
-  }
-  if (h->ev_lru && h->seen_lru != h->gen_lru) {
-    FI_CUDA(cudaStreamWaitEvent(h->s_pa, h->ev_lru, 0));
-    h->seen_lru = h->gen_lru;
-  }
-  if (h->part_seq >= 2) FI_CUDA(cudaStreamWaitEvent(h->s_pa, h->ev_a[s2], 0));
-  if (h->part_seq >= 3) FI_CUDA(cudaStreamWaitEvent(h->s_pa, h->ev_b3[s3], 0));
-  {
-    LaunchScope ls(h, h->s_pa, K_HASH);
-    // (the kernel also zeroes the request-queue counter of this batch's match_pick: one runtime call less per batch)
-    // hash_blocks runs as 4 persistent CTAs per SM here (FI_EPP_PIPE_HASH_CTAS / option "pipe_hash_ctas" overrides;
-    // a large value = one CTA per request).  With one CTA per request the step is bimodal: 116 us on most boxes,
-    // 138 us on others (among them the 8-GPU node) with the same binary — depending on which of the two kernels
-    // gets its CTAs resident first, hash_blocks' 16 384 short CTAs and match_pick's 324 long ones (80 registers
-    // x 256 threads x 3 per SM) lock each other out of the SMs.  Four hashing CTAs (32 K registers) always leave
-    // room for one matching CTA next to them: 122.6-123.3 us on both kinds of box.
-    const uint32_t hash_ctas = h->pipe_hash_ctas ? h->pipe_hash_ctas : 4u;
-    FI_CUDA(launch_hash_blocks(d_prompts, d_offsets, R, h->cfg.block_bytes, h->cfg.max_blocks, h->MP, pre, nb,
-                               hash_ctas * (uint32_t)h->part_main_sms, h->s_pa, h->d_work + 8 + s3));
-  }
-  FI_CUDA(cudaEventRecord(h->ev_h[s2], h->s_pa));
-  // ---- chain(k) on its own SMs: chain[s2] free once match(k-2) has read it
-  FI_CUDA(cudaStreamWaitEvent(h->s_pw, h->ev_h[s2], 0));
-  if (h->part_seq >= 2) FI_CUDA(cudaStreamWaitEvent(h->s_pw, h->ev_b3[(k + 1) % 3], 0));  // (k - 2) mod 3
-  {
-    LaunchScope ls(h, h->s_pw, K_CHAIN);
-    const bool compact = h->part_compact < 0 ? h->part_walk_sms < 24 : h->part_compact != 0;
-    FI_CUDA(launch_chain_finalize(pre, nb, d_h0, R, h->MP, chain, compact, h->s_pw));
-  }
-  FI_CUDA(cudaEventRecord(h->ev_a[s2], h->s_pw));
-  // ---- match(k): every submitted index op and pod-state update is visible
-  if (h->eps_dirty || h->lora_dirty) {
-    int rc = upload_endpoints(h);  // (on s_main)
-    if (rc != FI_OK) return rc;
-    rc = upload_lora(h);
-    if (rc != FI_OK) return rc;
-    FI_CUDA(cudaEventRecord(h->ev_up, h->s_main));
-    FI_CUDA(cudaStreamWaitEvent(h->s_pb, h->ev_up, 0));
-  }
-  if (h->seen_index != h->gen_index) {
-    FI_CUDA(cudaStreamWaitEvent(h->s_pb, h->ev_index, 0));
-    h->seen_index = h->gen_index;
-  }
-  FI_CUDA(cudaStreamWaitEvent(h->s_pb, h->ev_a[s2], 0));
-  MatchParams mp{};
-  fill_match_params(h, mp, chain, nb, d_offsets, d_h0, nullptr, R, d_out, true);
-  mp.work_counter = h->d_work + 8 + s3;
-  mp.max_ctas_per_sm = h->pipe_match_ctas;
-  mp.zero_work_counter = 0;  // hash_blocks of this batch did
-  {
-    LaunchScope ls(h, h->s_pb, K_MATCH);
-    FI_CUDA(launch_match_pick(mp, h->part_main_sms, h->s_pb));
-  }
-  FI_CUDA(cudaEventRecord(h->ev_b3[s3], h->s_pb));
-  h->ev_pick = h->ev_b3[s3];
-  h->pipe_seq++;
-  h->part_seq++;
-  h->stats.pick_calls++;
-  h->stats.requests += R;
-  return FI_OK;
-}
-
-// Pipelined device path: enqueue one batch.  Stage A on s_a, stage B on s_main (see fi_epp::s_a).
-int submit_pick(fi_epp* h, const uint8_t* d_prompts, const uint64_t* d_offsets, const uint64_t* d_h0, uint32_t R,
-                fi_pick* d_out, cudaStream_t us) {
-  int rc = flush_ops(h);
-  if (rc != FI_OK) return rc;
-  rc = check_counters(h);
-  if (rc != FI_OK) return rc;
-  if (!h->d_chain2) {
-    FI_CUDA(cudaMalloc(&h->d_chain2, (size_t)h->cfg.max_batch * h->MP * sizeof(uint64_t)));
-    FI_CUDA(cudaMalloc(&h->d_nblocks2, (size_t)h->cfg.max_batch * sizeof(uint32_t)));
-  }
-  setup_partition(h);
-  if (h->part_state == 1 && h->trace_call < 0) {
-    if (!h->part_active) {
-      // switching from the two-stream pipeline (or first use): everything in flight there is ordered before us
-      // through ev_plain / ev_pick; the slot events of the partitioned pipeline start fresh
-      FI_CUDA(cudaStreamWaitEvent(h->s_pa, h->ev_pick, 0));
-      FI_CUDA(cudaStreamWaitEvent(h->s_pw, h->ev_pick, 0));
-      h->part_active = true;
-      h->part_seq = 0;
-      h->seen_index = h->seen_plain = h->seen_lru = ~0ull;
-    }
-    return submit_pick_partitioned(h, d_prompts, d_offsets, d_h0, R, d_out, us);
-  }
-  // FI_EPP_TRACE=<call>: timeline of three consecutive pipelined batches (printed by fi_epp_pick_wait)
-  if (!h->profiling && h->trace_call >= 0 && (long)h->stats.pick_calls >= h->trace_call &&
-      (long)h->stats.pick_calls < h->trace_call + 3) {
-    if ((long)h->stats.pick_calls == h->trace_call) {
-      if (!h->ev_trace0) cudaEventCreate(&h->ev_trace0);
-      FI_CUDA(cudaStreamSynchronize(h->s_main));
-      FI_CUDA(cudaStreamSynchronize(h->s_a));
-      FI_CUDA(cudaEventRecord(h->ev_trace0, h->s_main));
-      FI_CUDA(cudaStreamWaitEvent(h->s_a, h->ev_trace0, 0));
-    }
-    h->tracing = true;
-  } else if (h->tracing && (long)h->stats.pick_calls >= h->trace_call + 3) {
-    h->tracing = false;  // events stay queued until the dump
-  }
-  const uint32_t slot = (uint32_t)(h->pipe_seq & 1);
-  uint64_t* chain = slot ? h->d_chain2 : h->d_chain;
-  uint32_t* nb = slot ? h->d_nblocks2 : h->d_nblocks;
-  // ---- stage A: inputs are ready in the caller's stream order; the slot's buffers are free once the
-  // match of two batches ago is done; d_pre is free once the previous plain pick (if any) is done
-  FI_CUDA(cudaEventRecord(h->ev_in, us));
-  FI_CUDA(cudaStreamWaitEvent(h->s_a, h->ev_in, 0));
-  if (h->pipe_seq >= 2) FI_CUDA(cudaStreamWaitEvent(h->s_a, h->ev_b[slot], 0));
-  FI_CUDA(cudaStreamWaitEvent(h->s_a, h->ev_plain, 0));
-  if (h->ev_lru) FI_CUDA(cudaStreamWaitEvent(h->s_a, h->ev_lru, 0));  // a device-LRU Add may still be reading d_chain
-  {
-    LaunchScope ls(h, h->s_a, K_HASH);
-    // The SM split of the pipeline: this batch's block hashing runs BESIDE the previous batch's match_pick —
-    // hash_blocks as at most pipe_hash_ctas CTAs per SM, match_pick as at most pipe_match_ctas (its three CTAs of
-    // 79 registers would leave no room) — instead of one after the other.
-    FI_CUDA(launch_hash_blocks(d_prompts, d_offsets, R, h->cfg.block_bytes, h->cfg.max_blocks, h->MP, h->d_pre, nb,
-                               h->pipe_hash_ctas * (uint32_t)h->sm_count, h->s_a));
-  }
-  // The chain walk is serial latency — a warp per scheduler that wants an issue slot every few cycles — and
-  // runs 3x slower next to a busy kernel (measured: 30 -> 100 us under match_pick), so it waits for the
-  // previous batch's match to drain; what overlaps is this batch's block hashing with that match.
-  if (h->pipe_seq >= 1) FI_CUDA(cudaStreamWaitEvent(h->s_a, h->ev_b[slot ^ 1u], 0));
-  {
-    LaunchScope ls(h, h->s_a, K_CHAIN);
-    FI_CUDA(launch_chain_finalize(h->d_pre, nb, d_h0, R, h->MP, chain, false, h->s_a));
-  }
-  FI_CUDA(cudaEventRecord(h->ev_a[slot], h->s_a));
-  // ---- stage B
-  FI_CUDA(cudaStreamWaitEvent(h->s_main, h->ev_index, 0));  // every submitted op is visible
-  rc = upload_endpoints(h);
-  if (rc != FI_OK) return rc;
-  rc = upload_lora(h);
-  if (rc != FI_OK) return rc;
-  FI_CUDA(cudaStreamWaitEvent(h->s_main, h->ev_a[slot], 0));
-  MatchParams mp{};
-  fill_match_params(h, mp, chain, nb, d_offsets, d_h0, nullptr, R, d_out, true);
-  mp.work_counter = h->d_work + 8 + slot;
-  mp.max_ctas_per_sm = h->pipe_match_ctas;
-  {
-    LaunchScope ls(h, h->s_main, K_MATCH);
-    FI_CUDA(launch_match_pick(mp, h->sm_count, h->s_main));
-  }
-  FI_CUDA(cudaEventRecord(h->ev_b[slot], h->s_main));
-  h->ev_pick = h->ev_pick_own;
-  FI_CUDA(cudaEventRecord(h->ev_pick, h->s_main));
-  h->pipe_seq++;
-  h->stats.pick_calls++;
-  h->stats.requests += R;
-  return FI_OK;
 }
 
 int validate_config(const fi_epp_config& c, std::string* err) {
@@ -1635,7 +60,7 @@ int validate_config(const fi_epp_config& c, std::string* err) {
   return FI_OK;
 }
 
-}  // namespace
+}  // namespace fi
 
 // =============================================================================
 // C ABI
@@ -1693,92 +118,24 @@ int fi_epp_model_seed(const void* model, size_t model_len, const void* salt, siz
 }
 
 void* fi_epp_pinned_alloc(size_t bytes) {
-  void* p = nullptr;
-  if (cudaMallocHost(&p, bytes ? bytes : 1) != cudaSuccess) return nullptr;
-  return p;
+  HostPtr<void> p;
+  if (host_alloc(p, bytes ? bytes : 1) != cudaSuccess) return nullptr;
+  return p.release();
 }
-void fi_epp_pinned_free(void* p) {
-  if (p) cudaFreeHost(p);
-}
+void fi_epp_pinned_free(void* p) { HostPtr<void> released_here(p); }
 
 const char* fi_epp_last_error(const fi_epp* h) { return h ? h->err.c_str() : "null handle"; }
 
+// Every resource of the handle has an owner that releases it; the order of the members of fi_epp is the order
+// of release.
 void fi_epp_destroy(fi_epp* h) {
   if (!h) return;
   cudaSetDevice(h->cfg.device);
-  if (h->s_main) cudaStreamSynchronize(h->s_main);
-  if (h->s_index) cudaStreamSynchronize(h->s_index);
-  if (h->comm && g_nccl.CommDestroy) g_nccl.CommDestroy(h->comm);
+  for (cudaStream_t s : {h->s_main.get(), h->s_index.get(), h->s_copy.get(), h->s_a.get()})
+    if (s) cudaStreamSynchronize(s);
+  if (h->part)
+    for (cudaStream_t s : {h->part->s_pw.get(), h->part->s_pa.get(), h->part->s_pb.get()}) cudaStreamSynchronize(s);
   drain_profile(h);
-  for (auto e : h->ev_pool) cudaEventDestroy(e);
-  cudaFree(h->d_prompts);
-  cudaFree(h->d_offsets);
-  cudaFree(h->d_h0);
-  cudaFree(h->d_pre);
-  cudaFree(h->d_chain);
-  cudaFree(h->d_nblocks);
-  cudaFree(h->d_picks);
-  cudaFree(h->d_local);
-  cudaFree(h->d_gather);
-  cudaFree(h->d_glog_n);
-  cudaFree(h->d_glog_a);
-  cudaFree(h->d_glog_v);
-  cudaFree(h->d_ghdr);
-  cudaFree(h->d_ggather);
-  if (h->h_ghdr) cudaFreeHost(h->h_ghdr);
-  for (int k = 0; k < FI_MAX_RANKS; ++k)
-    if (h->peer_ipc[k]) cudaIpcCloseMemHandle(h->peer_ipc[k]);
-  cudaFree(h->d_xchg);
-  if (h->h_xerr) cudaFreeHost((void*)h->h_xerr);
-  cudaFree(h->d_probed);
-  cudaFree(h->d_work);
-  cudaFree(h->d_ctr);
-  cudaFree(h->d_eps);
-  cudaFree(h->d_sc);
-  cudaFree(h->d_elig);
-  cudaFree(h->d_zero);
-  cudaFree(h->d_ztie);
-  cudaFree(h->d_lora);
-  cudaFree(h->d_adapters);
-  if (h->h_adapters) cudaFreeHost(h->h_adapters);
-  h->pool.reset();
-  h->lrus.clear();
-  h->lru_arena.release();
-  free_dev_lru(h);
-  cudaFree(h->d_lru_plan);
-  if (h->h_lru_plan) cudaFreeHost(h->h_lru_plan);
-  cudaFree(h->d_lru_chains);
-  free_index(h->ix);
-  free_index(h->ix_spare);
-  for (int b = 0; b < 2; ++b) {
-    cudaFree(h->d_sets[b]);
-    cudaFree(h->d_clears[b]);
-    if (h->h_sets[b]) cudaFreeHost(h->h_sets[b]);
-    if (h->h_clears[b]) cudaFreeHost(h->h_clears[b]);
-    if (h->ev_buf[b]) cudaEventDestroy(h->ev_buf[b]);
-  }
-  if (h->h_picks) cudaFreeHost(h->h_picks);
-  if (h->h_offsets) cudaFreeHost(h->h_offsets);
-  if (h->h_h0) cudaFreeHost(h->h_h0);
-  if (h->h_nblocks) cudaFreeHost(h->h_nblocks);
-  if (h->h_ctr) cudaFreeHost(h->h_ctr);
-  for (cudaEvent_t e : {h->ev_index, h->ev_user, h->ev_done, h->ev_ctr})
-    if (e) cudaEventDestroy(e);
-  for (int k = 0; k < fi_epp::kMaxFeedSlices; ++k)
-    if (h->ev_copy[k]) cudaEventDestroy(h->ev_copy[k]);
-  for (cudaEvent_t e : {h->ev_in, h->ev_a[0], h->ev_a[1], h->ev_b[0], h->ev_b[1], h->ev_pick_own, h->ev_plain})
-    if (e) cudaEventDestroy(e);
-  cudaFree(h->d_chain2);
-  cudaFree(h->d_nblocks2);
-  cudaFree(h->d_pre2);
-  cudaFree(h->d_nblocks3);
-  for (cudaEvent_t e : {h->ev_h[0], h->ev_h[1], h->ev_b3[0], h->ev_b3[1], h->ev_b3[2], h->ev_up})
-    if (e) cudaEventDestroy(e);
-  for (cudaStream_t st : {h->s_pw, h->s_pa, h->s_pb})
-    if (st) cudaStreamDestroy(st);
-  destroy_partition(h);
-  for (cudaStream_t s : {h->s_main, h->s_index, h->s_copy, h->s_a})
-    if (s) cudaStreamDestroy(s);
   delete h;
 }
 
@@ -1806,8 +163,7 @@ int fi_epp_create(const fi_epp_config* cfg, fi_epp** out) {
     return FI_ERR_INVALID;
   }
   auto die = [&](int rc) {
-    std::fprintf(stderr, "fi_epp_create: %s\n", h->err.c_str());
-    fi_epp_destroy(up.release());
+    std::fprintf(stderr, "fi_epp_create: %s\n", h->err.c_str());  // (`up` releases what was created)
     return rc;
   };
 #define FI_TRY(call)                                                    \
@@ -1848,59 +204,60 @@ int fi_epp_create(const fi_epp_config* cfg, fi_epp** out) {
     if (h->cfg.index_slots > 0x80000000ull) h->cfg.index_slots = 0x80000000ull;
   }
 
-  FI_TRY(cudaStreamCreateWithFlags(&h->s_main, cudaStreamNonBlocking));
-  FI_TRY(cudaStreamCreateWithFlags(&h->s_index, cudaStreamNonBlocking));
-  FI_TRY(cudaStreamCreateWithFlags(&h->s_copy, cudaStreamNonBlocking));
-  FI_TRY(cudaStreamCreateWithFlags(&h->s_a, cudaStreamNonBlocking));
-  for (cudaEvent_t* e : {&h->ev_in, &h->ev_a[0], &h->ev_a[1], &h->ev_b[0], &h->ev_b[1], &h->ev_pick_own, &h->ev_plain})
-    FI_TRY(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
-  h->ev_pick = h->ev_pick_own;
-  for (int k = 0; k < fi_epp::kMaxFeedSlices; ++k) FI_TRY(cudaEventCreateWithFlags(&h->ev_copy[k], cudaEventDisableTiming));
+  for (Stream* s : {&h->s_main, &h->s_index, &h->s_copy, &h->s_a}) {
+    cudaStream_t q = nullptr;
+    FI_TRY(cudaStreamCreateWithFlags(&q, cudaStreamNonBlocking));
+    s->reset(q);
+  }
+  for (Event* e : {&h->ev_in, &h->ev_a[0], &h->ev_a[1], &h->ev_b[0], &h->ev_b[1], &h->ev_pick_own, &h->ev_plain})
+    FI_TRY(event_create(*e));
+  h->ev_pick = h->ev_pick_own.get();
+  for (int k = 0; k < fi_epp::kMaxFeedSlices; ++k) FI_TRY(event_create(h->ev_copy[k]));
   if (const char* e = std::getenv("FI_EPP_FEED_SLICES")) {
     const long v = std::strtol(e, nullptr, 10);
     h->feed_slices = (uint32_t)std::min<long>(std::max<long>(v, 1), fi_epp::kMaxFeedSlices);
   }
-  for (cudaEvent_t* e : {&h->ev_index, &h->ev_user, &h->ev_done, &h->ev_ctr})
-    FI_TRY(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
-  FI_TRY(cudaEventRecord(h->ev_index, h->s_index));
+  for (Event* e : {&h->ev_index, &h->ev_user, &h->ev_done, &h->ev_ctr})
+    FI_TRY(event_create(*e));
+  FI_TRY(cudaEventRecord(h->ev_index.get(), h->s_index.get()));
   const uint64_t R = cfg->max_batch;
   // rows of the per-request buffers: whole groups of 32 requests (the pre-states are tiled), and — for a shard
   // of a bigger pool — room for the in-place all-gather of `world` equal slices of 32-aligned length
   h->chain_rows = (uint32_t)((R + 31) / 32 * 32);
   if (cfg->endpoint_count < cfg->num_endpoints) h->chain_rows += 32 * (FI_MAX_RANKS + 1);
   if (const char* e = std::getenv("FI_EPP_SHARD_HASH")) h->split_hash = std::strcmp(e, "split") == 0;
-  FI_TRY(cudaMalloc(&h->d_prompts, h->cfg.max_prompt_bytes + 64));
-  FI_TRY(cudaMalloc(&h->d_offsets, (R + 1) * sizeof(uint64_t)));
-  FI_TRY(cudaMalloc(&h->d_h0, R * sizeof(uint64_t)));
-  FI_TRY(cudaMalloc(&h->d_pre, (size_t)h->chain_rows * h->MP * sizeof(uint64_t)));
-  FI_TRY(cudaMalloc(&h->d_chain, (size_t)h->chain_rows * h->MP * sizeof(uint64_t)));
-  FI_TRY(cudaMalloc(&h->d_nblocks, (size_t)h->chain_rows * sizeof(uint32_t)));
-  FI_TRY(cudaMalloc(&h->d_picks, R * h->P * sizeof(fi_pick)));
-  FI_TRY(cudaMalloc(&h->d_probed, 8 * sizeof(unsigned long long)));
-  FI_TRY(cudaMemset(h->d_probed, 0, 8 * sizeof(unsigned long long)));
-  FI_TRY(cudaMalloc(&h->d_work, 16 * sizeof(uint32_t)));
-  FI_TRY(cudaMemset(h->d_work, 0, 16 * sizeof(uint32_t)));
-  FI_TRY(cudaMallocHost(&h->h_picks, R * h->P * sizeof(fi_pick)));
-  FI_TRY(cudaMallocHost(&h->h_offsets, (R + 1) * sizeof(uint64_t)));
-  FI_TRY(cudaMallocHost(&h->h_h0, R * sizeof(uint64_t)));
-  FI_TRY(cudaMallocHost(&h->h_nblocks, R * sizeof(uint32_t)));
+  FI_TRY(dev_alloc(h->d_prompts, h->cfg.max_prompt_bytes + 64));
+  FI_TRY(dev_alloc(h->d_offsets, (R + 1) * sizeof(uint64_t)));
+  FI_TRY(dev_alloc(h->d_h0, R * sizeof(uint64_t)));
+  FI_TRY(dev_alloc(h->d_pre, (size_t)h->chain_rows * h->MP * sizeof(uint64_t)));
+  FI_TRY(dev_alloc(h->d_chain, (size_t)h->chain_rows * h->MP * sizeof(uint64_t)));
+  FI_TRY(dev_alloc(h->d_nblocks, (size_t)h->chain_rows * sizeof(uint32_t)));
+  FI_TRY(dev_alloc(h->d_picks, R * h->P * sizeof(fi_pick)));
+  FI_TRY(dev_alloc(h->d_probed, 8 * sizeof(unsigned long long)));
+  FI_TRY(cudaMemset(h->d_probed.get(), 0, 8 * sizeof(unsigned long long)));
+  FI_TRY(dev_alloc(h->d_work, 16 * sizeof(uint32_t)));
+  FI_TRY(cudaMemset(h->d_work.get(), 0, 16 * sizeof(uint32_t)));
+  FI_TRY(host_alloc(h->h_picks, R * h->P * sizeof(fi_pick)));
+  FI_TRY(host_alloc(h->h_offsets, (R + 1) * sizeof(uint64_t)));
+  FI_TRY(host_alloc(h->h_h0, R * sizeof(uint64_t)));
+  FI_TRY(host_alloc(h->h_nblocks, R * sizeof(uint32_t)));
 
   // index
-  FI_TRY(cudaMalloc(&h->d_ctr, sizeof(IndexCounters)));
-  FI_TRY(cudaMemset(h->d_ctr, 0, sizeof(IndexCounters)));
-  FI_TRY(cudaMallocHost(&h->h_ctr, sizeof(IndexCounters)));
-  std::memset(h->h_ctr, 0, sizeof(IndexCounters));
+  FI_TRY(dev_alloc(h->d_ctr, sizeof(IndexCounters)));
+  FI_TRY(cudaMemset(h->d_ctr.get(), 0, sizeof(IndexCounters)));
+  FI_TRY(host_alloc(h->h_ctr, sizeof(IndexCounters)));
+  std::memset(h->h_ctr.get(), 0, sizeof(IndexCounters));
   {
     int rc = alloc_index(h, h->cfg.index_slots, &h->ix);
     if (rc != FI_OK) return die(rc);
   }
   for (int b = 0; b < 2; ++b) {
-    FI_TRY(cudaMallocHost(&h->h_sets[b], kOpChunk * sizeof(fi_index_op)));
-    FI_TRY(cudaMallocHost(&h->h_clears[b], kOpChunk * sizeof(fi_index_op)));
-    FI_TRY(cudaMalloc(&h->d_sets[b], kOpChunk * sizeof(fi_index_op)));
-    FI_TRY(cudaMalloc(&h->d_clears[b], kOpChunk * sizeof(fi_index_op)));
-    FI_TRY(cudaEventCreateWithFlags(&h->ev_buf[b], cudaEventDisableTiming));
-    FI_TRY(cudaEventRecord(h->ev_buf[b], h->s_index));
+    FI_TRY(host_alloc(h->h_sets[b], kOpChunk * sizeof(fi_index_op)));
+    FI_TRY(host_alloc(h->h_clears[b], kOpChunk * sizeof(fi_index_op)));
+    FI_TRY(dev_alloc(h->d_sets[b], kOpChunk * sizeof(fi_index_op)));
+    FI_TRY(dev_alloc(h->d_clears[b], kOpChunk * sizeof(fi_index_op)));
+    FI_TRY(event_create(h->ev_buf[b]));
+    FI_TRY(cudaEventRecord(h->ev_buf[b].get(), h->s_index.get()));
   }
   if (cfg->lru_capacity) {
     // virtual reservation only: an endpoint's tables become resident when it is first touched
@@ -1911,26 +268,26 @@ int fi_epp_create(const fi_epp_config* cfg, fi_epp** out) {
   // endpoints + score tables
   h->eps.assign(cfg->num_endpoints, EndpointDev{0.0, 0, 0, 0, 0});
   const uint32_t Epad = h->W * 32;
-  FI_TRY(cudaMalloc(&h->d_eps, (size_t)cfg->num_endpoints * sizeof(EndpointDev)));
-  FI_TRY(cudaMalloc(&h->d_sc, (size_t)FI_EPP_MAX_PROFILES * FI_EPP_MAX_SCORERS * Epad * sizeof(double)));
-  FI_TRY(cudaMalloc(&h->d_elig, (size_t)FI_EPP_MAX_PROFILES * h->W * sizeof(uint32_t)));
-  FI_TRY(cudaMalloc(&h->d_zero, FI_EPP_MAX_PROFILES * sizeof(ZeroBest)));
-  FI_TRY(cudaMalloc(&h->d_ztie, (size_t)FI_EPP_MAX_PROFILES * h->W * sizeof(uint32_t)));
-  FI_TRY(cudaMemset(h->d_ztie, 0, (size_t)FI_EPP_MAX_PROFILES * h->W * sizeof(uint32_t)));
-  FI_TRY(cudaMemset(h->d_sc, 0, (size_t)FI_EPP_MAX_PROFILES * FI_EPP_MAX_SCORERS * Epad * sizeof(double)));
-  FI_TRY(cudaMemset(h->d_elig, 0, (size_t)FI_EPP_MAX_PROFILES * h->W * sizeof(uint32_t)));
+  FI_TRY(dev_alloc(h->d_eps, (size_t)cfg->num_endpoints * sizeof(EndpointDev)));
+  FI_TRY(dev_alloc(h->d_sc, (size_t)FI_EPP_MAX_PROFILES * FI_EPP_MAX_SCORERS * Epad * sizeof(double)));
+  FI_TRY(dev_alloc(h->d_elig, (size_t)FI_EPP_MAX_PROFILES * h->W * sizeof(uint32_t)));
+  FI_TRY(dev_alloc(h->d_zero, FI_EPP_MAX_PROFILES * sizeof(ZeroBest)));
+  FI_TRY(dev_alloc(h->d_ztie, (size_t)FI_EPP_MAX_PROFILES * h->W * sizeof(uint32_t)));
+  FI_TRY(cudaMemset(h->d_ztie.get(), 0, (size_t)FI_EPP_MAX_PROFILES * h->W * sizeof(uint32_t)));
+  FI_TRY(cudaMemset(h->d_sc.get(), 0, (size_t)FI_EPP_MAX_PROFILES * FI_EPP_MAX_SCORERS * Epad * sizeof(double)));
+  FI_TRY(cudaMemset(h->d_elig.get(), 0, (size_t)FI_EPP_MAX_PROFILES * h->W * sizeof(uint32_t)));
   h->st.n_profiles = h->P;
   h->st.Epad = Epad;
-  h->st.sc = h->d_sc;
-  h->st.elig = h->d_elig;
-  h->st.zero = h->d_zero;
-  h->st.ztie = h->d_ztie;
+  h->st.sc = h->d_sc.get();
+  h->st.elig = h->d_elig.get();
+  h->st.zero = h->d_zero.get();
+  h->st.ztie = h->d_ztie.get();
   h->lora.assign(Epad, LoraDev{});
-  FI_TRY(cudaMalloc(&h->d_lora, (size_t)Epad * sizeof(LoraDev)));
-  FI_TRY(cudaMemset(h->d_lora, 0, (size_t)Epad * sizeof(LoraDev)));
-  FI_TRY(cudaMalloc(&h->d_adapters, R * sizeof(uint64_t)));
-  FI_TRY(cudaMallocHost(&h->h_adapters, R * sizeof(uint64_t)));
-  h->st.lora = h->d_lora;
+  FI_TRY(dev_alloc(h->d_lora, (size_t)Epad * sizeof(LoraDev)));
+  FI_TRY(cudaMemset(h->d_lora.get(), 0, (size_t)Epad * sizeof(LoraDev)));
+  FI_TRY(dev_alloc(h->d_adapters, R * sizeof(uint64_t)));
+  FI_TRY(host_alloc(h->h_adapters, R * sizeof(uint64_t)));
+  h->st.lora = h->d_lora.get();
   h->st.has_lora = 0;
   for (uint32_t p = 0; p < h->P; ++p)
     for (uint32_t s = 0; s < cfg->profiles[p].n_scorers; ++s)
@@ -1946,7 +303,7 @@ int fi_epp_create(const fi_epp_config* cfg, fi_epp** out) {
       d.weight[s] = (double)cfg->profiles[p].scorers[s].weight;
     }
   }
-  FI_TRY(cudaStreamSynchronize(h->s_index));
+  FI_TRY(cudaStreamSynchronize(h->s_index.get()));
   FI_TRY(cudaDeviceSynchronize());
 #undef FI_TRY
   *out = up.release();
@@ -1994,624 +351,18 @@ int fi_epp_endpoints_lora_update(fi_epp* h, const fi_endpoint_lora* s, uint32_t 
   return FI_OK;
 }
 
-// One collective index update of a sharded pool = `rounds` gossip rounds on every rank; `step(i)` stages and
-// flushes this rank's share of round i (nothing if it has fewer).  Single rank: just the steps.
-static int run_rounds(fi_epp* h, uint64_t mine, int my_err, const std::function<int(uint64_t)>& step) {
-  if (h->world <= 1) {
-    if (my_err != FI_OK) return my_err;
-    for (uint64_t i = 0; i < mine; ++i) {
-      int rc = step(i);
-      if (rc != FI_OK) return rc;
-    }
-    return FI_OK;
-  }
-  // a rank whose arguments were rejected still takes part (with zero rounds) so that the others do not hang
-  uint64_t rounds = 0;
-  int rc = agree_rounds(h, my_err == FI_OK ? mine : 0, &rounds);
-  if (rc != FI_OK) return rc;
-  for (uint64_t i = 0; i < rounds; ++i) {
-    if (my_err == FI_OK && i < mine) {
-      rc = step(i);
-      if (rc != FI_OK) return rc;
-    }
-    rc = gossip_round(h);
-    if (rc != FI_OK) return rc;
-  }
-  return my_err;
-}
-
-int fi_epp_index_apply(fi_epp* h, const fi_index_op* ops, uint64_t n) {
-  if (!h || (!ops && n)) return FI_ERR_INVALID;
-  std::lock_guard<std::mutex> lk(h->mu);
-  if (cudaSetDevice(h->cfg.device) != cudaSuccess) return fail(h, FI_ERR_CUDA, "cudaSetDevice failed");
-  int err = check_counters(h);
-  for (uint64_t i = 0; i < n && err == FI_OK; ++i) {
-    if (ops[i].op != FI_OP_SET && ops[i].op != FI_OP_CLEAR) err = fail(h, FI_ERR_INVALID, "bad index opcode");
-    else if (ops[i].endpoint >= h->cfg.num_endpoints) err = fail(h, FI_ERR_INVALID, "index op endpoint out of range");
-  }
-  const uint32_t lo = h->cfg.endpoint_begin, cnt = h->cfg.endpoint_count;
-  // rounds of kOpChunk input ops: a round never overflows the staging buffers (or, sharded, the gossip log)
-  const uint64_t rounds = (n + kOpChunk - 1) / kOpChunk;
-  return run_rounds(h, rounds, err, [&](uint64_t i) -> int {
-    const uint64_t i0 = i * kOpChunk, i1 = std::min(n, i0 + kOpChunk);
-    for (uint64_t k = i0; k < i1; ++k) {
-      const fi_index_op& op = ops[k];
-      if (op.endpoint - lo >= cnt) continue;  // another rank's shard
-      int rc = submit_op(h, op.hash, op.endpoint, op.op);
-      if (rc != FI_OK) return rc;
-    }
-    return flush_ops(h);
-  });
-}
-
-int fi_epp_index_add_chain(fi_epp* h, uint32_t endpoint, const uint64_t* hashes, uint32_t n) {
-  if (!h || (!hashes && n)) return FI_ERR_INVALID;
-  std::lock_guard<std::mutex> lk(h->mu);
-  if (cudaSetDevice(h->cfg.device) != cudaSuccess) return fail(h, FI_ERR_CUDA, "cudaSetDevice failed");
-  if (!h->cfg.lru_capacity) return fail(h, FI_ERR_STATE, "lru_capacity is 0: the host LRU is disabled");
-  if (h->world > 1) return fail(h, FI_ERR_STATE, "sharded pool: use the collective fi_epp_index_add_chains");  // (device LRU too)
-  if (endpoint >= h->cfg.num_endpoints) return fail(h, FI_ERR_INVALID, "endpoint out of range");
-  const uint32_t e = endpoint - h->cfg.endpoint_begin;
-  if (e >= h->cfg.endpoint_count) return FI_OK;  // another rank's shard
-  int rc = choose_lru_mode(h);
-  if (rc != FI_OK) return rc;
-  if (h->lru_mode == 1) return lru_device_add(h, &endpoint, hashes, false, n, &n, 1);
-  rc = check_counters(h);
-  if (rc != FI_OK) return rc;
-  LruSet& l = h->lrus[e];
-  for (uint32_t i = 0; i < n; ++i) {
-    uint64_t ev = 0;
-    bool did = false;
-    const bool inserted = l.touch(hashes[i], &ev, &did);
-    if (did) {
-      rc = submit_op(h, ev, endpoint, FI_OP_CLEAR);
-      if (rc != FI_OK) return rc;
-    }
-    if (inserted) {
-      rc = submit_op(h, hashes[i], endpoint, FI_OP_SET);
-      if (rc != FI_OK) return rc;
-    }
-  }
-  // the deltas stay staged: they are launched when the staging buffer fills and, at the latest,
-  // by the next pick / sync (one launch group per batch of decisions instead of one per chain)
-  return FI_OK;
-}
-
-namespace {
-
-struct CopyJob {
-  fi_index_op* dst;
-  const fi_index_op* src;
-  size_t n;
-};
-
-}  // namespace
-
-// Upstream PreRequest for a whole batch of decisions: indexer.Add(chain_r, endpoints[r]) for r = 0..R-1, in
-// request order per endpoint (the endpoints' LRUs are independent of each other, so they are walked in
-// parallel on the host worker pool; the result equals R sequential fi_epp_index_add_chain calls).
-int fi_epp_index_add_chains(fi_epp* h, const uint32_t* endpoints, const uint64_t* chains, uint32_t pitch_blocks,
-                            const uint32_t* nblocks, uint32_t R) {
-  if (!h || ((!endpoints || !chains || !nblocks) && R)) return FI_ERR_INVALID;
-  std::lock_guard<std::mutex> lk(h->mu);
-  if (cudaSetDevice(h->cfg.device) != cudaSuccess) return fail(h, FI_ERR_CUDA, "cudaSetDevice failed");
-  int err = FI_OK;
-  if (!h->cfg.lru_capacity) err = fail(h, FI_ERR_STATE, "lru_capacity is 0: the host LRU is disabled");
-  for (uint32_t r = 0; r < R && err == FI_OK; ++r) {
-    if (endpoints[r] != FI_NO_ENDPOINT && endpoints[r] >= h->cfg.num_endpoints) err = fail(h, FI_ERR_INVALID, "endpoint out of range");
-    else if (nblocks[r] > pitch_blocks) err = fail(h, FI_ERR_INVALID, "nblocks[r] larger than the chain pitch");
-  }
-  if (err == FI_OK) err = choose_lru_mode(h);
-  if (err == FI_OK && h->lru_mode == 1) return lru_device_add(h, endpoints, chains, false, pitch_blocks, nblocks, R);
-  if (err == FI_OK) err = check_counters(h);
-
-  // ---- 1./2. bucket the requests by endpoint and walk the LRUs on the worker pool (lru_batch.h)
-  const uint32_t lo = h->cfg.endpoint_begin, EL = h->cfg.endpoint_count;
-  std::vector<WorkerOps>& outs = h->lru_outs;  // persistent: capacity survives from batch to batch
-  size_t nseg = 0;
-  const auto t_start = std::chrono::steady_clock::now();
-  if (!h->pool) {
-    unsigned t = std::min(usable_cores(), 128u);
-    if (const char* ev = std::getenv("FI_EPP_LRU_THREADS")) t = (unsigned)std::max(1L, std::strtol(ev, nullptr, 10));
-    if (h->lru_threads) t = h->lru_threads;
-    h->pool.reset(new WorkerPool(t));
-  }
-  if (err == FI_OK) nseg = lru_walk_batch(h->lrus, lo, EL, endpoints, chains, pitch_blocks, nblocks, R, *h->pool, outs);
-  else for (auto& o : outs) o.begin_batch();
-  const auto t_walked = std::chrono::steady_clock::now();
-
-  // ---- 3. stage segment by segment (SETs, then CLEARs), flushing whenever a staging buffer is full.
-  // `flushes` is first counted (dry run) so that the ranks of a sharded pool can agree on the rounds.
-  std::vector<CopyJob> jobs;
-  auto run_jobs = [&]() {
-    if (jobs.empty()) return;
-    // big copies into the pinned staging buffers go through the worker pool
-    std::vector<CopyJob> pieces;
-    const size_t kPiece = 1u << 16;
-    for (const CopyJob& j : jobs)
-      for (size_t o = 0; o < j.n; o += kPiece) pieces.push_back(CopyJob{j.dst + o, j.src + o, std::min(kPiece, j.n - o)});
-    h->pool->run((uint32_t)pieces.size(), [&](uint32_t t, unsigned) {
-      std::memcpy(pieces[t].dst, pieces[t].src, pieces[t].n * sizeof(fi_index_op));
-    });
-    jobs.clear();
-  };
-  // walk(dry): returns the number of flushes; !dry performs them through do_flush
-  auto walk = [&](bool dry, const std::function<int()>& do_flush, uint64_t* n_flush) -> int {
-    uint64_t ns = dry ? 0 : h->n_sets, nc = dry ? 0 : h->n_clears, flushes = 0;
-    auto flush = [&]() -> int {
-      ++flushes;
-      if (!dry) {
-        run_jobs();
-        h->n_sets = ns;
-        h->n_clears = nc;
-        int rc = do_flush();
-        if (rc != FI_OK) return rc;
-      }
-      ns = nc = 0;
-      return FI_OK;
-    };
-    for (size_t seg = 0; seg < nseg; ++seg) {
-      for (int kind = 0; kind < 2; ++kind) {
-        for (auto& o : outs) {
-          if (o.nseg <= seg) continue;
-          const std::vector<fi_index_op>& v = kind == 0 ? o.sets[seg] : o.clears[seg];
-          size_t done = 0;
-          while (done < v.size()) {
-            uint64_t& fillc = kind == 0 ? ns : nc;
-            const size_t room = (size_t)(kOpChunk - fillc);
-            const size_t take = std::min(room, v.size() - done);
-            if (!dry && take) {
-              fi_index_op* base = kind == 0 ? h->h_sets[h->cur_buf] : h->h_clears[h->cur_buf];
-              jobs.push_back(CopyJob{base + fillc, v.data() + done, take});
-            }
-            fillc += take;
-            done += take;
-            if (fillc == kOpChunk) {
-              int rc = flush();
-              if (rc != FI_OK) return rc;
-            }
-          }
-        }
-      }
-      if (seg + 1 < nseg && (ns || nc)) {  // segment boundary: the next segment's SETs must run after these CLEARs
-        int rc = flush();
-        if (rc != FI_OK) return rc;
-      }
-    }
-    if (!dry) {
-      run_jobs();
-      h->n_sets = ns;
-      h->n_clears = nc;
-    }
-    if (n_flush) *n_flush = flushes;
-    return FI_OK;
-  };
-
-  if (h->world <= 1) {
-    if (err != FI_OK) return err;
-    // the tail stays staged: it is launched with the next flush — at the latest by the next pick / sync
-    int rc1 = walk(false, [&]() { return flush_ops(h); }, nullptr);
-    if (h->verbose) {
-      const auto t_end = std::chrono::steady_clock::now();
-      size_t nops = 0;
-      for (auto& o : outs)
-        for (size_t sg = 0; sg < o.nseg; ++sg) nops += o.sets[sg].size() + o.clears[sg].size();
-      std::fprintf(stderr, "[fi_epp] add_chains: %u requests, %zu ops, %zu segment(s), %u workers: LRU walk %.2f ms, staging %.2f ms\n",
-                   R, nops, nseg, h->pool->size(), std::chrono::duration<double, std::milli>(t_walked - t_start).count(),
-                   std::chrono::duration<double, std::milli>(t_end - t_walked).count());
-    }
-    return rc1;
-  }
-  // sharded: every flush is one gossip round, the tail included
-  uint64_t mine = 0;
-  if (err == FI_OK) {
-    walk(true, nullptr, &mine);
-    mine += 1;  // the tail
-  }
-  uint64_t rounds = 0;
-  int rc = agree_rounds(h, err == FI_OK ? mine : 0, &rounds);
-  if (rc != FI_OK) return rc;
-  uint64_t did = 0;
-  if (err == FI_OK) {
-    rc = walk(false, [&]() -> int {
-      int r2 = flush_ops(h);
-      if (r2 != FI_OK) return r2;
-      ++did;
-      return gossip_round(h);
-    }, nullptr);
-    if (rc != FI_OK) return rc;
-    rc = flush_ops(h);  // the tail
-    if (rc != FI_OK) return rc;
-  }
-  for (; did < rounds; ++did) {
-    rc = gossip_round(h);
-    if (rc != FI_OK) return rc;
-  }
-  return err;
-}
-
-// The same with the chains already in device memory (e.g. the chains_out of fi_epp_pick_batch_device): nothing
-// but the two small host arrays crosses PCIe.  Device LRU only.
-int fi_epp_index_add_chains_device(fi_epp* h, const uint32_t* endpoints, const void* d_chains, uint32_t pitch_blocks,
-                                   const uint32_t* nblocks, uint32_t R, void* stream) {
-  if (!h || ((!endpoints || !nblocks) && R)) return FI_ERR_INVALID;
-  std::lock_guard<std::mutex> lk(h->mu);
-  if (cudaSetDevice(h->cfg.device) != cudaSuccess) return fail(h, FI_ERR_CUDA, "cudaSetDevice failed");
-  if (!h->cfg.lru_capacity) return fail(h, FI_ERR_STATE, "lru_capacity is 0: no LRU");
-  if (!d_chains) {  // the chains of the handle's most recent stream-ordered pick, still in its own buffer
-    if (R > h->last_plain_R) return fail(h, FI_ERR_STATE, "no pick batch of that size to take the chains from");
-    d_chains = h->d_chain;
-    pitch_blocks = h->MP;
-  }
-  for (uint32_t r = 0; r < R; ++r) {
-    if (endpoints[r] != FI_NO_ENDPOINT && endpoints[r] >= h->cfg.num_endpoints) return fail(h, FI_ERR_INVALID, "endpoint out of range");
-    if (nblocks[r] > pitch_blocks) return fail(h, FI_ERR_INVALID, "nblocks[r] larger than the chain pitch");
-  }
-  int rc = choose_lru_mode(h);
-  if (rc != FI_OK) return rc;
-  if (h->lru_mode != 1) return fail(h, FI_ERR_STATE, "fi_epp_index_add_chains_device needs the device LRU");
-  // the chains were produced on the caller's stream
-  FI_CUDA(cudaEventRecord(h->ev_user, (cudaStream_t)stream));
-  FI_CUDA(cudaStreamWaitEvent(h->s_index, h->ev_user, 0));
-  return lru_device_add(h, endpoints, static_cast<const uint64_t*>(d_chains), true, pitch_blocks, nblocks, R);
-}
-
-// Diagnostics: the device LRU's content for one endpoint, least recently used first.
-int fi_epp_lru_dump(fi_epp* h, uint32_t endpoint, uint64_t* out, uint32_t cap, uint32_t* n_out) {
-  if (!h || !n_out || (!out && cap)) return FI_ERR_INVALID;
-  std::lock_guard<std::mutex> lk(h->mu);
-  if (cudaSetDevice(h->cfg.device) != cudaSuccess) return fail(h, FI_ERR_CUDA, "cudaSetDevice failed");
-  *n_out = 0;
-  const uint32_t e = endpoint - h->cfg.endpoint_begin;
-  if (e >= h->cfg.endpoint_count) return fail(h, FI_ERR_INVALID, "endpoint outside this handle's shard");
-  if (h->lru_mode != 1 || !h->dlru_ready) return h->lru_mode == 0 ? fail(h, FI_ERR_STATE, "the handle runs the host LRU") : FI_OK;
-  uint64_t* d_out = nullptr;
-  uint32_t* d_n = nullptr;
-  FI_CUDA(cudaMalloc(&d_out, ((size_t)h->dlru.capacity + 1) * sizeof(uint64_t)));
-  if (cudaMalloc(&d_n, sizeof(uint32_t)) != cudaSuccess) {
-    cudaFree(d_out);
-    return fail(h, FI_ERR_NOMEM, "cudaMalloc failed");
-  }
-  uint32_t n = 0;
-  cudaError_t er = launch_lru_dump(h->dlru, e, d_out, d_n, h->s_index);
-  if (er == cudaSuccess) er = cudaMemcpyAsync(&n, d_n, sizeof(n), cudaMemcpyDeviceToHost, h->s_index);
-  if (er == cudaSuccess) er = cudaStreamSynchronize(h->s_index);
-  if (er == cudaSuccess && n) er = cudaMemcpy(out, d_out, (size_t)std::min(n, cap) * sizeof(uint64_t), cudaMemcpyDeviceToHost);
-  cudaFree(d_out);
-  cudaFree(d_n);
-  if (er != cudaSuccess) return fail(h, FI_ERR_CUDA, cudaGetErrorString(er));
-  *n_out = n;
-  return FI_OK;
-}
-
-// Diagnostics: totals of the device-resident LRU since create — out[0] SETs emitted, [1] CLEARs emitted,
-// [2] doomed winners, [3] endpoint maintenance passes, [4] requests deferred to a conservative pass, [5] sub-batches.
-int fi_epp_lru_counters(fi_epp* h, uint64_t out[6]) {
-  if (!h || !out) return FI_ERR_INVALID;
-  std::lock_guard<std::mutex> lk(h->mu);
-  if (cudaSetDevice(h->cfg.device) != cudaSuccess) return fail(h, FI_ERR_CUDA, "cudaSetDevice failed");
-  for (int i = 0; i < 6; ++i) out[i] = 0;
-  if (h->lru_mode != 1 || !h->dlru_ready) return FI_OK;
-  FI_CUDA(cudaStreamSynchronize(h->s_index));
-  out[0] = h->h_lru_stat->n_sets;
-  out[1] = h->h_lru_stat->n_clears;
-  out[2] = h->h_lru_stat->n_doomed;
-  out[3] = h->h_lru_stat->n_maintained;
-  out[4] = h->lru_deferred;
-  out[5] = h->lru_sub_batches;
-  return FI_OK;
-}
-
-int fi_epp_index_sync(fi_epp* h) {
-  if (!h) return FI_ERR_INVALID;
-  std::lock_guard<std::mutex> lk(h->mu);
-  if (cudaSetDevice(h->cfg.device) != cudaSuccess) return fail(h, FI_ERR_CUDA, "cudaSetDevice failed");
-  int rc = flush_ops(h);
-  if (rc != FI_OK) return rc;
-  FI_CUDA(cudaStreamSynchronize(h->s_index));
-  return check_counters(h);
-}
-
-int fi_epp_index_stats(fi_epp* h, fi_index_stats* out) {
-  if (!h || !out) return FI_ERR_INVALID;
-  std::lock_guard<std::mutex> lk(h->mu);
-  if (cudaSetDevice(h->cfg.device) != cudaSuccess) return fail(h, FI_ERR_CUDA, "cudaSetDevice failed");
-  int rc = flush_ops(h);
-  if (rc != FI_OK) return rc;
-  FI_CUDA(cudaStreamSynchronize(h->s_index));
-  IndexCounters c;
-  FI_CUDA(cudaMemcpy(&c, h->d_ctr, sizeof(c), cudaMemcpyDeviceToHost));
-  out->slots = h->ix.C;
-  out->used = c.used;
-  out->tombstones = c.tombstones;
-  out->rebuilds = h->rebuilds;
-  out->ops_applied = h->ops_applied;
-  uint64_t l = 0;
-  if (h->lru_mode == 1 && h->dlru_ready) {
-    std::vector<uint32_t> cnt(h->dlru.EL);
-    FI_CUDA(cudaMemcpy(cnt.data(), h->dlru.count, cnt.size() * sizeof(uint32_t), cudaMemcpyDeviceToHost));
-    for (uint32_t c2 : cnt) l += c2;
-    out->ops_applied += h->h_lru_stat->n_sets + h->h_lru_stat->n_clears;
-  } else {
-    for (auto& s : h->lrus) l += s.size();
-  }
-  out->lru_entries = l;
-  return FI_OK;
-}
-
-// diagnostics for tests: out[i] = 1 iff (ops[i].endpoint, ops[i].hash) is in the GPU index
-int fi_epp_index_contains(fi_epp* h, const fi_index_op* q, uint64_t n, uint8_t* out) {
-  if (!h || (!q && n) || (!out && n)) return FI_ERR_INVALID;
-  std::lock_guard<std::mutex> lk(h->mu);
-  if (cudaSetDevice(h->cfg.device) != cudaSuccess) return fail(h, FI_ERR_CUDA, "cudaSetDevice failed");
-  int rc = flush_ops(h);
-  if (rc != FI_OK) return rc;
-  if (n == 0) return FI_OK;
-  fi_index_op* dq = nullptr;
-  uint8_t* dout = nullptr;
-  FI_CUDA(cudaMalloc(&dq, n * sizeof(fi_index_op)));
-  if (cudaMalloc(&dout, n) != cudaSuccess) {
-    cudaFree(dq);
-    return fail(h, FI_ERR_NOMEM, "cudaMalloc failed");
-  }
-  cudaError_t e = cudaMemcpyAsync(dq, q, n * sizeof(fi_index_op), cudaMemcpyHostToDevice, h->s_index);
-  if (e == cudaSuccess) {
-    LaunchScope ls(h, h->s_index, K_OTHER);
-    e = launch_index_contains(h->ix, dq, n, h->cfg.endpoint_begin, h->cfg.endpoint_count, dout, h->s_index);
-  }
-  if (e == cudaSuccess) e = cudaMemcpyAsync(out, dout, n, cudaMemcpyDeviceToHost, h->s_index);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(h->s_index);
-  cudaFree(dq);
-  cudaFree(dout);
-  if (e != cudaSuccess) return fail(h, FI_ERR_CUDA, cudaGetErrorString(e));
-  return FI_OK;
-}
-
-static int check_batch(fi_epp* h, const uint64_t* offsets, uint32_t R, uint64_t* total) {
-  if (R > h->cfg.max_batch) return fail(h, FI_ERR_CAPACITY, "batch larger than max_batch");
-  if (offsets[0] != 0) return fail(h, FI_ERR_INVALID, "offsets[0] must be 0");
-  for (uint32_t r = 0; r < R; ++r)
-    if (offsets[r + 1] < offsets[r]) return fail(h, FI_ERR_INVALID, "offsets must be non-decreasing");
-  *total = offsets[R];
-  if (*total > h->cfg.max_prompt_bytes) return fail(h, FI_ERR_CAPACITY, "prompt bytes larger than max_prompt_bytes");
-  return FI_OK;
-}
-
-static int stage_inputs(fi_epp* h, const uint8_t* prompts, const uint64_t* offsets, const uint64_t* h0, uint32_t R,
-                        uint64_t total, bool copy_prompts = true) {
-  std::memcpy(h->h_offsets, offsets, (size_t)(R + 1) * sizeof(uint64_t));
-  std::memcpy(h->h_h0, h0, (size_t)R * sizeof(uint64_t));
-  FI_CUDA(cudaMemcpyAsync(h->d_offsets, h->h_offsets, (size_t)(R + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, h->s_main));
-  FI_CUDA(cudaMemcpyAsync(h->d_h0, h->h_h0, (size_t)R * sizeof(uint64_t), cudaMemcpyHostToDevice, h->s_main));
-  if (total && copy_prompts) {
-    FI_CUDA(cudaMemcpyAsync(h->d_prompts, prompts, total, cudaMemcpyHostToDevice, h->s_main));
-    h->stats.h2d_bytes += total;
-  }
-  h->stats.h2d_bytes += (size_t)(2 * R + 1) * sizeof(uint64_t);
-  return FI_OK;
-}
-
-static int copy_chains_out(fi_epp* h, uint64_t* chains_out, uint32_t R, cudaMemcpyKind kind, cudaStream_t s) {
-  const size_t row = (size_t)h->cfg.max_blocks * sizeof(uint64_t);
-  FI_CUDA(cudaMemcpy2DAsync(chains_out, row, h->d_chain, (size_t)h->MP * sizeof(uint64_t), row, R, kind, s));
-  if (kind == cudaMemcpyDeviceToHost) h->stats.d2h_bytes += row * R;
-  return FI_OK;
-}
-
-int fi_epp_hash_batch(fi_epp* h, const uint8_t* prompts, const uint64_t* offsets, const uint64_t* h0, uint32_t R,
-                      uint64_t* chains_out, uint32_t* nblocks_out) {
-  if (!h || !offsets || (!h0 && R) || (!prompts && R && offsets[R])) return FI_ERR_INVALID;
-  std::lock_guard<std::mutex> lk(h->mu);
-  if (cudaSetDevice(h->cfg.device) != cudaSuccess) return fail(h, FI_ERR_CUDA, "cudaSetDevice failed");
-  if (R == 0) return FI_OK;
-  uint64_t total = 0;
-  int rc = check_batch(h, offsets, R, &total);
-  if (rc != FI_OK) return rc;
-  rc = stage_inputs(h, prompts, offsets, h0, R, total);
-  if (rc != FI_OK) return rc;
-  if (h->pipe_seq)  // a pipelined batch's stage A (on s_a) shares d_pre with us
-    FI_CUDA(cudaStreamWaitEvent(h->s_main, h->ev_a[(h->pipe_seq - 1) & 1], 0));
-  if (h->ev_lru) FI_CUDA(cudaStreamWaitEvent(h->s_main, h->ev_lru, 0));  // a device-LRU Add may still be reading d_chain
-  h->last_plain_R = 0;  // d_chain no longer holds a pick batch's chains
-  rc = run_hash(h, h->d_prompts, h->d_offsets, h->d_h0, 0, R, h->s_main);
-  if (rc != FI_OK) return rc;
-  if (chains_out) {
-    rc = copy_chains_out(h, chains_out, R, cudaMemcpyDeviceToHost, h->s_main);
-    if (rc != FI_OK) return rc;
-  }
-  if (nblocks_out) {
-    FI_CUDA(cudaMemcpyAsync(h->h_nblocks, h->d_nblocks, (size_t)R * sizeof(uint32_t), cudaMemcpyDeviceToHost, h->s_main));
-    h->stats.d2h_bytes += (size_t)R * sizeof(uint32_t);
-  }
-  FI_CUDA(cudaStreamSynchronize(h->s_main));
-  if (nblocks_out) std::memcpy(nblocks_out, h->h_nblocks, (size_t)R * sizeof(uint32_t));
-  return FI_OK;
-}
-
-int fi_epp_pick_batch(fi_epp* h, const uint8_t* prompts, const uint64_t* offsets, const uint64_t* h0, uint32_t R,
-                      fi_pick* out, uint64_t* chains_out) {
-  return fi_epp_pick_batch_lora(h, prompts, offsets, h0, nullptr, R, out, chains_out);
-}
-
-int fi_epp_pick_batch_lora(fi_epp* h, const uint8_t* prompts, const uint64_t* offsets, const uint64_t* h0,
-                           const uint64_t* adapters, uint32_t R, fi_pick* out, uint64_t* chains_out) {
-  if (!h || !offsets || (!h0 && R) || (!out && R) || (!prompts && R && offsets[R])) return FI_ERR_INVALID;
-  std::lock_guard<std::mutex> lk(h->mu);
-  if (cudaSetDevice(h->cfg.device) != cudaSuccess) return fail(h, FI_ERR_CUDA, "cudaSetDevice failed");
-  if (R == 0) return FI_OK;
-  uint64_t total = 0;
-  int rc = check_batch(h, offsets, R, &total);
-  if (rc != FI_OK) return rc;
-  rc = stage_inputs(h, prompts, offsets, h0, R, total, /*copy_prompts=*/false);  // run_pick feeds the prompts
-  if (rc != FI_OK) return rc;
-  if (adapters) {
-    std::memcpy(h->h_adapters, adapters, (size_t)R * sizeof(uint64_t));
-    FI_CUDA(cudaMemcpyAsync(h->d_adapters, h->h_adapters, (size_t)R * sizeof(uint64_t), cudaMemcpyHostToDevice, h->s_main));
-    h->stats.h2d_bytes += (size_t)R * sizeof(uint64_t);
-  }
-  const HostFeed feed{prompts, offsets};
-  rc = run_pick(h, h->d_prompts, h->d_offsets, h->d_h0, adapters ? h->d_adapters : nullptr, R, h->d_picks, &feed);
-  if (rc != FI_OK) return rc;
-  const size_t pb = (size_t)R * h->P * sizeof(fi_pick);
-  FI_CUDA(cudaMemcpyAsync(h->h_picks, h->d_picks, pb, cudaMemcpyDeviceToHost, h->s_main));
-  h->stats.d2h_bytes += pb;
-  if (chains_out) {
-    rc = copy_chains_out(h, chains_out, R, cudaMemcpyDeviceToHost, h->s_main);
-    if (rc != FI_OK) return rc;
-  }
-  FI_CUDA(cudaStreamSynchronize(h->s_main));
-  if (h->h_xerr && *h->h_xerr) {  // reported once; the tags are monotonic, so later steps can succeed again
-    *h->h_xerr = 0;
-    return fail(h, FI_ERR_COMM, "peer exchange timed out waiting for another rank");
-  }
-  std::memcpy(out, h->h_picks, pb);
-  return FI_OK;
-}
-
-int fi_epp_pick_batch_device(fi_epp* h, const void* d_prompts, const void* d_offsets, const void* d_h0, uint32_t R,
-                             uint64_t total_prompt_bytes, void* d_out, void* d_chains_out, void* stream) {
-  return fi_epp_pick_batch_device_lora(h, d_prompts, d_offsets, d_h0, nullptr, R, total_prompt_bytes, d_out, d_chains_out,
-                                       stream);
-}
-
-int fi_epp_pick_batch_device_lora(fi_epp* h, const void* d_prompts, const void* d_offsets, const void* d_h0,
-                                  const void* d_adapters, uint32_t R, uint64_t total_prompt_bytes, void* d_out,
-                                  void* d_chains_out, void* stream) {
-  if (!h || !d_offsets || (!d_h0 && R) || (!d_out && R)) return FI_ERR_INVALID;
-  std::lock_guard<std::mutex> lk(h->mu);
-  if (cudaSetDevice(h->cfg.device) != cudaSuccess) return fail(h, FI_ERR_CUDA, "cudaSetDevice failed");
-  if (R == 0) return FI_OK;
-  if (R > h->cfg.max_batch) return fail(h, FI_ERR_CAPACITY, "batch larger than max_batch");
-  (void)total_prompt_bytes;  // inputs stay where they are: no staging copy, no capacity limit
-  cudaStream_t us = (cudaStream_t)stream;
-  FI_CUDA(cudaEventRecord(h->ev_user, us));
-  FI_CUDA(cudaStreamWaitEvent(h->s_main, h->ev_user, 0));
-  int rc = run_pick(h, (const uint8_t*)d_prompts, (const uint64_t*)d_offsets, (const uint64_t*)d_h0,
-                    (const uint64_t*)d_adapters, R, (fi_pick*)d_out);
-  if (rc != FI_OK) return rc;
-  if (d_chains_out) {
-    rc = copy_chains_out(h, (uint64_t*)d_chains_out, R, cudaMemcpyDeviceToDevice, h->s_main);
-    if (rc != FI_OK) return rc;
-  }
-  FI_CUDA(cudaEventRecord(h->ev_done, h->s_main));
-  FI_CUDA(cudaStreamWaitEvent(us, h->ev_done, 0));
-  return FI_OK;
-}
-
-int fi_epp_pick_submit(fi_epp* h, const void* d_prompts, const void* d_offsets, const void* d_h0, uint32_t R,
-                       uint64_t total_prompt_bytes, void* d_out, void* stream) {
-  if (!h || !d_offsets || (!d_h0 && R) || (!d_out && R)) return FI_ERR_INVALID;
-  bool plain;
-  {
-    std::lock_guard<std::mutex> lk(h->mu);
-    plain = h->world > 1 || !h->fast_hash;  // sharded pools and odd block sizes: the stream-ordered path
-  }
-  if (plain) return fi_epp_pick_batch_device(h, d_prompts, d_offsets, d_h0, R, total_prompt_bytes, d_out, nullptr, stream);
-  std::lock_guard<std::mutex> lk(h->mu);
-  if (cudaSetDevice(h->cfg.device) != cudaSuccess) return fail(h, FI_ERR_CUDA, "cudaSetDevice failed");
-  if (R == 0) return FI_OK;
-  if (R > h->cfg.max_batch) return fail(h, FI_ERR_CAPACITY, "batch larger than max_batch");
-  return submit_pick(h, (const uint8_t*)d_prompts, (const uint64_t*)d_offsets, (const uint64_t*)d_h0, R, (fi_pick*)d_out,
-                     (cudaStream_t)stream);
-}
-
-// out[0] = 1 if the pipelined path (fi_epp_pick_submit) runs on a partitioned GPU, out[1] / out[2] = SMs of the chain-walk
-// partition / of the hashing + matching partition (0 when unpartitioned or not yet used).
-int fi_epp_pipeline_info(fi_epp* h, int32_t out[3]) {
-  if (!h || !out) return FI_ERR_INVALID;
-  std::lock_guard<std::mutex> lk(h->mu);
-  out[0] = h->part_state == 1 ? 1 : 0;
-  out[1] = h->part_state == 1 ? h->part_walk_sms : 0;
-  out[2] = h->part_state == 1 ? h->part_main_sms : 0;
-  return FI_OK;
-}
-
-int fi_epp_pick_wait(fi_epp* h, void* stream) {
-  if (!h) return FI_ERR_INVALID;
-  std::lock_guard<std::mutex> lk(h->mu);
-  if (cudaSetDevice(h->cfg.device) != cudaSuccess) return fail(h, FI_ERR_CUDA, "cudaSetDevice failed");
-  FI_CUDA(cudaStreamWaitEvent((cudaStream_t)stream, h->ev_pick, 0));  // s_main runs the batches in order
-  if (!h->profiling && !h->pending_ev.empty() && h->ev_trace0) {
-    h->tracing = true;
-    dump_trace(h, 0);
-  }
-  return FI_OK;
-}
-
-int fi_epp_comm_unique_id(uint8_t out[FI_EPP_UNIQUE_ID_BYTES]) {
-  if (!out) return FI_ERR_INVALID;
-  std::lock_guard<std::mutex> lk(g_nccl_mu);
-  std::string e;
-  if (!g_nccl.load(&e)) {
-    std::fprintf(stderr, "fi_epp_comm_unique_id: %s\n", e.c_str());
-    return FI_ERR_COMM;
-  }
-  ncclUniqueId id;
-  if (g_nccl.GetUniqueId(&id) != ncclSuccess) return FI_ERR_COMM;
-  static_assert(sizeof(ncclUniqueId) == FI_EPP_UNIQUE_ID_BYTES, "unique id size");
-  std::memcpy(out, &id, sizeof(id));
-  return FI_OK;
-}
-
-int fi_epp_comm_init(fi_epp* h, const uint8_t id_bytes[FI_EPP_UNIQUE_ID_BYTES], uint32_t rank, uint32_t world) {
-  if (!h || !id_bytes || world == 0 || rank >= world) return FI_ERR_INVALID;
-  std::lock_guard<std::mutex> lk(h->mu);
-  if (cudaSetDevice(h->cfg.device) != cudaSuccess) return fail(h, FI_ERR_CUDA, "cudaSetDevice failed");
-  if (h->comm) return fail(h, FI_ERR_STATE, "communicator already initialised");
-  if (world > 32) return fail(h, FI_ERR_INVALID, "more than 32 ranks: the directory keeps one presence bit per rank");
-  if (h->ops_applied || h->n_sets || h->n_clears)
-    return fail(h, FI_ERR_STATE, "fi_epp_comm_init must precede the first index update (the directory is built by gossip)");
-  if (world == 1) {
-    h->rank = 0;
-    h->world = 1;
-    return FI_OK;
-  }
-  {
-    std::lock_guard<std::mutex> lk2(g_nccl_mu);
-    std::string e;
-    if (!g_nccl.load(&e)) return fail(h, FI_ERR_COMM, e);
-  }
-  ncclUniqueId id;
-  std::memcpy(&id, id_bytes, sizeof(id));
-  int rc = g_nccl.CommInitRank(&h->comm, (int)world, id, (int)rank);
-  if (rc != ncclSuccess) {
-    h->comm = nullptr;
-    return fail(h, FI_ERR_COMM, std::string("ncclCommInitRank: ") + (g_nccl.GetErrorString ? g_nccl.GetErrorString(rc) : "error"));
-  }
-  const uint64_t R = h->cfg.max_batch;
-  FI_CUDA(cudaMalloc(&h->d_local, R * h->P * sizeof(fi_pick)));
-  FI_CUDA(cudaMalloc(&h->d_gather, (size_t)world * R * h->P * sizeof(fi_pick)));
-  // directory gossip (index_kernels.cu): this rank's transition log + gather buffers
-  FI_CUDA(cudaMalloc(&h->d_glog_n, 2 * sizeof(unsigned long long)));
-  FI_CUDA(cudaMemset(h->d_glog_n, 0, 2 * sizeof(unsigned long long)));
-  FI_CUDA(cudaMalloc(&h->d_glog_a, kOpChunk * sizeof(uint64_t)));
-  FI_CUDA(cudaMalloc(&h->d_glog_v, kOpChunk * sizeof(uint64_t)));
-  FI_CUDA(cudaMalloc(&h->d_ghdr, (size_t)(world + 1) * 2 * sizeof(unsigned long long)));
-  FI_CUDA(cudaMallocHost(&h->h_ghdr, (size_t)(world + 1) * 2 * sizeof(unsigned long long)));
-  FI_CUDA(cudaMalloc(&h->d_ggather, (size_t)world * kOpChunk * sizeof(uint64_t)));
-  h->rank = rank;
-  h->world = world;
-  return setup_peer_exchange(h);
-}
-
-int fi_epp_comm_exchange(fi_epp* h) {
-  if (!h) return FI_ERR_INVALID;
-  std::lock_guard<std::mutex> lk(h->mu);
-  if (h->world <= 1) return FI_EXCHANGE_NONE;
-  return h->px.enabled ? FI_EXCHANGE_PEER : FI_EXCHANGE_NCCL;
-}
-
 int fi_epp_set_option(fi_epp* h, const char* name, int64_t value) {
   if (!h || !name) return FI_ERR_INVALID;
   std::lock_guard<std::mutex> lk(h->mu);
   const std::string n(name);
   if (n == "exchange") {
     if (h->world <= 1) return fail(h, FI_ERR_STATE, "exchange: not a sharded pool");
+    PeerXchg& px = h->shard->px;
     if (value == FI_EXCHANGE_NCCL) {
-      h->px.enabled = 0;
+      px.enabled = 0;
     } else if (value == FI_EXCHANGE_PEER) {
-      if (!h->px.base[h->rank == 0 ? 1 : 0]) return fail(h, FI_ERR_STATE, "exchange: the peers' buffers were never mapped");
-      h->px.enabled = 1;
+      if (!px.base[h->rank == 0 ? 1 : 0]) return fail(h, FI_ERR_STATE, "exchange: the peers' buffers were never mapped");
+      px.enabled = 1;
     } else {
       return fail(h, FI_ERR_INVALID, "exchange: FI_EXCHANGE_PEER or FI_EXCHANGE_NCCL");
     }
@@ -2639,23 +390,23 @@ int fi_epp_set_option(fi_epp* h, const char* name, int64_t value) {
   }
   if (n == "pipe_partition") {
     if (value < 0 || value > 64) return fail(h, FI_ERR_INVALID, "pipe_partition: 0 (off) or the walker partition's SM count");
-    if (h->part_state == 1 && value == 0) {
-      // back to the unpartitioned pipeline (contexts are released with the handle); nothing of the partitioned
-      // one may still be in flight: the two share the pre-state / chain buffers
+    if (h->part && value == 0) {
+      // back to the unpartitioned pipeline, and the partition is released; nothing of the partitioned pipeline may
+      // still be in flight: the two share the pre-state / chain buffers
       cudaSetDevice(h->cfg.device);
-      for (cudaStream_t st : {h->s_pa, h->s_pw, h->s_pb})
-        if (st) cudaStreamSynchronize(st);
-      h->part_state = -1;
+      for (cudaStream_t st : {h->part->s_pa.get(), h->part->s_pw.get(), h->part->s_pb.get()}) cudaStreamSynchronize(st);
+      h->ev_pick = h->ev_pick_own.get();  // (it may name a slot event of the partition; those picks are done)
+      h->part.reset();
       h->part_active = false;
-    } else if (h->part_state != 1) {
+    } else if (!h->part) {
       h->part_want = (int)value;
-      h->part_state = 0;
+      h->part_tried = false;
     }
     return FI_OK;
   }
   if (n == "lru_table_slots") {
     if (value < 0 || value > (1ll << 30)) return fail(h, FI_ERR_INVALID, "lru_table_slots: 0 .. 2^30");
-    if (h->dlru_ready) return fail(h, FI_ERR_STATE, "lru_table_slots: the device LRU is already allocated");
+    if (h->dlru) return fail(h, FI_ERR_STATE, "lru_table_slots: the device LRU is already allocated");
     h->lru_table_slots = (uint32_t)value;
     return FI_OK;
   }
@@ -2683,9 +434,9 @@ int fi_epp_get_stats(fi_epp* h, fi_epp_stats* out) {
   if (cudaSetDevice(h->cfg.device) != cudaSuccess) return fail(h, FI_ERR_CUDA, "cudaSetDevice failed");
   drain_profile(h);
   if (h->profiling) {
-    FI_CUDA(cudaStreamSynchronize(h->s_main));
+    FI_CUDA(cudaStreamSynchronize(h->s_main.get()));
     unsigned long long pb[8] = {0};
-    FI_CUDA(cudaMemcpy(pb, h->d_probed, sizeof(pb), cudaMemcpyDeviceToHost));
+    FI_CUDA(cudaMemcpy(pb, h->d_probed.get(), sizeof(pb), cudaMemcpyDeviceToHost));
     h->stats.probed_blocks = pb[0];
     if (pb[5] && h->verbose)  // FI_MATCH_TIMING build: where a request's time goes inside match_pick
       std::fprintf(stderr, "[fi_epp] match_pick phases, cycles per request over %llu requests: stage %.0f, first lookup %.0f, "
@@ -2701,8 +452,8 @@ int fi_epp_reset_stats(fi_epp* h) {
   std::lock_guard<std::mutex> lk(h->mu);
   cudaSetDevice(h->cfg.device);
   drain_profile(h);
-  cudaStreamSynchronize(h->s_main);
-  cudaMemset(h->d_probed, 0, 8 * sizeof(unsigned long long));
+  cudaStreamSynchronize(h->s_main.get());
+  cudaMemset(h->d_probed.get(), 0, 8 * sizeof(unsigned long long));
   h->stats = fi_epp_stats{};
   return FI_OK;
 }

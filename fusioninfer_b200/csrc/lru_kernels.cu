@@ -17,7 +17,7 @@
 // in between.
 //
 // Capacity.  A table takes the batch's distinct keys on top of its C entries; it holds 0.85 TS, with TS between
-// 4 C and 32 C slots depending on how much HBM is free (engine.cu: a B200 gives 1 024 endpoints 1 Mi slots each).
+// 4 C and 32 C slots depending on how much HBM is free (engine_lru.cu: a B200 gives 1 024 endpoints 1 Mi slots each).
 // An endpoint that receives more NEW distinct keys than that in a single batch is detected while inserting
 // (slots are reserved before they are claimed), its touches are rolled back and its requests are re-run in
 // sub-batches of at most C touches, which always fit (lru_plan.h; endpoints are independent of each other, so
